@@ -3,7 +3,7 @@
 -> 6-connected CCL -> marching-cubes meshing at mip 2) on a synthetic 2048^3
 uint32 segmentation resident in HBM, one z-slab of the dataset per GPU.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--size S] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--size S] [--impl reference] [--dump-outputs DIR]
 
 Contract (see the task brief): W untimed warm-up steps, exactly K timed steps
 bracketed by barrier + device synchronisation, CUDA-event timing on the stream
@@ -250,27 +250,33 @@ def cpu_baseline_sample(pipe, ctx, budget_s=20.0):
 
 
 # ------------------------------------------------------------ parity self-check
+def read_box(ctx, dptr, shape, size, dtype, origin=(0, 0, 0)):
+  """Host copy of the `size` box at `origin` of a Fortran-order device volume of `shape`."""
+  from igneous_b200 import _shim
+  d = ctx.alloc(int(np.prod(size)) * np.dtype(dtype).itemsize)
+  _shim.check(ctx.lib.ign_copy_box_dev(ctx.handle, _shim.ptr(dptr), c.c_int(_shim.dtype_code(dtype)),
+                                       c.c_uint64(shape[0]), c.c_uint64(shape[1]), c.c_uint64(shape[2]),
+                                       c.c_uint64(origin[0]), c.c_uint64(origin[1]), c.c_uint64(origin[2]),
+                                       c.c_uint64(size[0]), c.c_uint64(size[1]), c.c_uint64(size[2]), _shim.ptr(d)))
+  h = ctx.to_host(d, size, dtype)
+  d.free()
+  return h
+
+
 def parity_check(ctx, pipe):
   """Untimed check of the benchmark's own products against the CPU oracle (run once after the
   timed loop, at the benchmark's full size): a 256x256x64 sub-box of the mips (bit-exact), the
   CCL labels of the same sub-box (every oracle component carries exactly one label, two
   components share a label only when they hold the same input id, 0 <-> 0) and every fragment
   of one MeshTask body on a 129x129x65 cutout of the mesh mip (bit-exact vertices and faces)."""
-  from igneous_b200 import _shim, zmesh
+  from igneous_b200 import zmesh
   from oracle import oracle as O
   O.build()
   sx, sy, sz = pipe.shape
   bx, by, bz = min(sx, 256), min(sy, 256), min(sz, 64)
 
   def box(dptr, shape, size, dtype):
-    d = ctx.alloc(int(np.prod(size)) * np.dtype(dtype).itemsize)
-    _shim.check(ctx.lib.ign_copy_box_dev(ctx.handle, _shim.ptr(dptr), c.c_int(_shim.dtype_code(dtype)),
-                                         c.c_uint64(shape[0]), c.c_uint64(shape[1]), c.c_uint64(shape[2]),
-                                         c.c_uint64(0), c.c_uint64(0), c.c_uint64(0), c.c_uint64(size[0]),
-                                         c.c_uint64(size[1]), c.c_uint64(size[2]), _shim.ptr(d)))
-    h = ctx.to_host(d, size, dtype)
-    d.free()
-    return h
+    return read_box(ctx, dptr, shape, size, dtype)
 
   out = {}
   seg = box(pipe.d_in, pipe.shape, (bx, by, bz), np.uint32)
@@ -309,6 +315,38 @@ def parity_check(ctx, pipe):
   out["mesh"] = ("ok (%d fragments bit-exact)" % n_lab) if ok else "MISMATCH"
   out["status"] = "ok" if all(v.startswith("ok") for v in out.values()) else "FAILED"
   return out
+
+
+DUMP_BOXES, DUMP_BOX = 32, (64, 64, 16)
+MESH_COUNTS = ("tasks", "triangles_in", "vertices_in", "triangles", "vertices", "label_fragments")
+
+
+def dump_outputs(ctx, pipe, out_dir):
+  """--dump-outputs: what the last timed step left behind, as float64 .npy files (exact for every
+  uint32 value), so that two builds can be compared output for output on the same inputs.
+
+    mip<k>.npy          [DUMP_BOXES, *DUMP_BOX] sample of mode-pooled mip k
+    ccl_labels.npy      [DUMP_BOXES, *DUMP_BOX] sample of the 6-connected CCL labels at mip 0
+    ccl_components.npy  [1] number of components
+    mesh_counts.npy     the MESH_COUNTS totals of the MeshTask bodies (the step keeps no fragments)
+
+  The volumes are far larger than a dump should be, so each is sampled as DUMP_BOXES boxes (clamped
+  to the volume) whose origins come from numpy's default_rng(0): the same boxes on every run with
+  the same --size.  At most 48 MiB in all."""
+  os.makedirs(out_dir, exist_ok=True)
+  u = np.random.default_rng(0).random((DUMP_BOXES, 3))
+
+  def sample(dptr, shape, dtype):
+    size = tuple(min(b, s) for b, s in zip(DUMP_BOX, shape))
+    origins = (u * (np.asarray(shape) - np.asarray(size) + 1)).astype(np.int64)
+    return np.stack([read_box(ctx, dptr, shape, size, dtype, o) for o in origins]).astype(np.float64)
+
+  for k, (dptr, shape) in enumerate(zip(pipe.d_mips, pipe.mip_shapes)):
+    np.save(os.path.join(out_dir, "mip%d.npy" % (k + 1)), sample(dptr, shape, pipe.dtype))
+  np.save(os.path.join(out_dir, "ccl_labels.npy"), sample(pipe.d_cc, pipe.shape, pipe.ccl_out_dtype))
+  np.save(os.path.join(out_dir, "ccl_components.npy"), np.array([pipe.n_components], dtype=np.float64))
+  np.save(os.path.join(out_dir, "mesh_counts.npy"),
+          np.array([pipe.mesh_stats[k] for k in MESH_COUNTS], dtype=np.float64))
 
 
 def multigpu_check(ctx, group, rank, world, dist):
@@ -476,7 +514,13 @@ def main():
                   help="download the labels into the input host buffer (forced automatically when host RAM is tight)")
   ap.add_argument("--simplify", type=int, default=None, help="simplification factor (default 100)")
   ap.add_argument("--mesh-streams", type=int, default=8, help="concurrent MeshTask bodies per GPU")
+  ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                  help="after the timed steps, write a fixed sample of the last step's products to DIR/<name>.npy")
   args = ap.parse_args()
+  if args.steps < 1:
+    ap.error("--steps must be at least 1")
+  if args.dump_outputs and (args.impl != "b200" or args.config != "headline"):
+    ap.error("--dump-outputs applies to the headline pipeline (--impl b200 --config headline)")
   if args.warmup < 3 and args.impl == "b200":
     args.warmup = 3
 
@@ -625,6 +669,8 @@ def main():
     "roofline": roofline, "clocks": clocks,
   }
 
+  if args.dump_outputs and rank == 0:  # before the e2e leg, which recomputes into the same buffers
+    dump_outputs(ctx, pipe, args.dump_outputs)
   if not args.no_parity_check:
     line["parity_check"] = parity_check(ctx, pipe) if rank == 0 else None
   if args.check and world > 1:
