@@ -16,9 +16,13 @@
 // byte-identical:
 //   1  k_cseg_scan<T, false>  one warp per block: the distinct values are extracted in
 //      ascending order (repeated warp minimum) -> n, bits, 64-bit hash of the table
-//   2  radix sort of (hash, block) -> the first block of every group of identical tables owns it
-//   3  exclusive scan of the per-block sizes -> offsets
-//   4  k_cseg_scan<T, true>   the same extraction again, now writing indices, tables, headers
+//   2  radix sort of (hash, block): blocks with equal tables are adjacent, in raster order
+//   3  k_cseg_owner  one warp per block compares its table with the earlier blocks of its hash
+//      group (first the group's head) -> owner = the first block in raster order with an EQUAL
+//      table.  The hash only groups; blocks whose tables differ but hash alike never share.
+//   4  exclusive scan of the per-block sizes -> offsets; the largest table offset is checked
+//      against the format's 24-bit limit with the total, in the one host sync of the encoder
+//   5  k_cseg_scan<T, true>   the same extraction again, now writing indices, tables, headers
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
 
@@ -45,6 +49,44 @@ __device__ __forceinline__ uint32_t cs_bits(uint32_t n) {
   return b;
 }
 
+// Loads block b into a warp: lane l holds block positions l, l+32, ... (position
+// p = (z*by + y)*bx + x).  Returns the slots inside the volume (bit k: slot k).
+template <typename T, int CS_PER_LANE>
+__device__ __forceinline__ uint32_t cs_load(const T* __restrict__ in, const CsegDims& d, uint64_t b, uint32_t lane,
+                                            uint64_t (&val)[CS_PER_LANE]) {
+  const uint32_t gxx = (uint32_t)(b % d.gx), gyy = (uint32_t)((b / d.gx) % d.gy), gzz = (uint32_t)(b / ((uint64_t)d.gx * d.gy));
+  const uint32_t x0 = gxx * d.bx, y0 = gyy * d.by, z0 = gzz * d.bz;
+  uint32_t have = 0;
+#pragma unroll
+  for (int k = 0; k < CS_PER_LANE; k++) {
+    const uint32_t p = lane + 32 * k;
+    val[k] = 0;
+    if (p < d.bvox) {
+      const uint32_t x = p % d.bx, y = (p / d.bx) % d.by, z = p / (d.bx * d.by);
+      if (x0 + x < d.sx && y0 + y < d.sy && z0 + z < d.sz) {
+        val[k] = (uint64_t)in[(x0 + x) + (uint64_t)d.sx * ((y0 + y) + (uint64_t)d.sy * (z0 + z))];
+        have |= 1u << k;
+      }
+    }
+  }
+  return have;
+}
+
+// warp minimum of the values in the slots of `todo` (~0ull when no lane has any)
+template <int CS_PER_LANE>
+__device__ __forceinline__ uint64_t cs_warp_min(const uint64_t (&val)[CS_PER_LANE], uint32_t todo) {
+  uint64_t m = ~0ull;
+#pragma unroll
+  for (int k = 0; k < CS_PER_LANE; k++)
+    if ((todo >> k) & 1u) m = val[k] < m ? val[k] : m;
+#pragma unroll
+  for (int s = 16; s > 0; s >>= 1) {
+    const uint64_t o = cs_shfl_xor(m, s);
+    m = o < m ? o : m;
+  }
+  return m;
+}
+
 // One warp per block.  WRITE = false: info[b] = {n, bits}, hash[b].  WRITE = true: the stream.
 template <typename T, bool WRITE, int CS_PER_LANE>  // CS_PER_LANE * 32 >= voxels per block
 __global__ void __launch_bounds__(128)
@@ -55,40 +97,18 @@ __global__ void __launch_bounds__(128)
   const uint32_t lane = threadIdx.x & 31u;
   const uint64_t b = (blockIdx.x * (uint64_t)blockDim.x + threadIdx.x) >> 5;
   if (b >= nblock) return;
-  const uint32_t gxx = (uint32_t)(b % d.gx), gyy = (uint32_t)((b / d.gx) % d.gy), gzz = (uint32_t)(b / ((uint64_t)d.gx * d.gy));
-  const uint32_t x0 = gxx * d.bx, y0 = gyy * d.by, z0 = gzz * d.bz;
-  // lane l holds block positions l, l+32, ... (position p = (z*by + y)*bx + x)
   uint64_t val[CS_PER_LANE];
   uint32_t idx[CS_PER_LANE];
-  uint32_t have = 0, todo = 0;  // bit k: slot k is inside the volume / not classified yet
+  const uint32_t have = cs_load<T, CS_PER_LANE>(in, d, b, lane, val);  // bit k: slot k is inside the volume
+  uint32_t todo = have;                                                 // bit k: slot k is not classified yet
 #pragma unroll
-  for (int k = 0; k < CS_PER_LANE; k++) {
-    const uint32_t p = lane + 32 * k;
-    val[k] = 0;
-    idx[k] = 0;
-    if (p < d.bvox) {
-      const uint32_t x = p % d.bx, y = (p / d.bx) % d.by, z = p / (d.bx * d.by);
-      if (x0 + x < d.sx && y0 + y < d.sy && z0 + z < d.sz) {
-        val[k] = (uint64_t)in[(x0 + x) + (uint64_t)d.sx * ((y0 + y) + (uint64_t)d.sy * (z0 + z))];
-        have |= 1u << k;
-      }
-    }
-  }
-  todo = have;
+  for (int k = 0; k < CS_PER_LANE; k++) idx[k] = 0;
   uint32_t n = 0;
   uint64_t h = 0x9E3779B97F4A7C15ull;
   const uint32_t toff = WRITE ? tab_off[b] : 0u;
   const bool own = WRITE ? (owner[b] == (uint32_t)b) : false;
   while (__any_sync(CS_FULL, todo != 0)) {
-    uint64_t m = ~0ull;
-#pragma unroll
-    for (int k = 0; k < CS_PER_LANE; k++)
-      if ((todo >> k) & 1u) m = val[k] < m ? val[k] : m;
-#pragma unroll
-    for (int s = 16; s > 0; s >>= 1) {
-      const uint64_t o = cs_shfl_xor(m, s);
-      m = o < m ? o : m;
-    }
+    const uint64_t m = cs_warp_min<CS_PER_LANE>(val, todo);
 #pragma unroll
     for (int k = 0; k < CS_PER_LANE; k++)
       if (((todo >> k) & 1u) && val[k] == m) {
@@ -143,18 +163,58 @@ __global__ void __launch_bounds__(256) k_iota32(uint32_t* p, uint32_t n) {
   if (i < n) p[i] = i;
 }
 
-// sorted (hash, block): the head of every run of equal hashes owns the table (the sort is stable
-// and the blocks entered it in ascending order, so the head is the smallest block of the run)
+// Do blocks a and b have equal tables?  Both must hold the same number of distinct values: their
+// ascending values are extracted in lock step (warp minimum) and compared, stopping at the first
+// difference.  Warp-uniform: every lane of the warp calls it with the same a, b.
+template <typename T, int CS_PER_LANE>
+__device__ __forceinline__ bool cs_same_table(const T* __restrict__ in, const CsegDims& d, uint64_t a, uint64_t b,
+                                              uint32_t lane) {
+  uint64_t va[CS_PER_LANE], vb[CS_PER_LANE];
+  uint32_t ta = cs_load<T, CS_PER_LANE>(in, d, a, lane, va);
+  uint32_t tb = cs_load<T, CS_PER_LANE>(in, d, b, lane, vb);
+  while (__any_sync(CS_FULL, ta != 0)) {
+    const uint64_t ma = cs_warp_min<CS_PER_LANE>(va, ta), mb = cs_warp_min<CS_PER_LANE>(vb, tb);
+    if (ma != mb) return false;
+#pragma unroll
+    for (int k = 0; k < CS_PER_LANE; k++) {
+      if (((ta >> k) & 1u) && va[k] == ma) ta &= ~(1u << k);
+      if (((tb >> k) & 1u) && vb[k] == mb) tb &= ~(1u << k);
+    }
+  }
+  return true;
+}
+
+// sorted (hash, block): heads of the runs of equal hashes (the sort is stable and the blocks
+// entered it in ascending order, so a run lists its blocks in raster order)
 __global__ void __launch_bounds__(256)
     k_cseg_heads(const unsigned long long* __restrict__ shash, uint32_t n, uint32_t* __restrict__ headpos) {
   const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n) headpos[i] = (i == 0 || shash[i - 1] != shash[i]) ? i : 0u;
 }
-__global__ void __launch_bounds__(256)
-    k_cseg_owner(const uint32_t* __restrict__ headpos, const uint32_t* __restrict__ sblock, uint32_t n,
+
+// One warp per sorted position i (block sblock[i]; headpos: inclusive max-scan of the head
+// positions).  Every block with a table equal to it sits in the same run, so the first block of
+// the run with an equal table is the first in raster order: it owns the table.  Without a hash
+// collision that is the head, one comparison; a run that mixes tables costs one comparison per
+// distinct table before the block's own.
+template <typename T, int CS_PER_LANE>
+__global__ void __launch_bounds__(128)
+    k_cseg_owner(const T* __restrict__ in, CsegDims d, const uint32_t* __restrict__ headpos,
+                 const uint32_t* __restrict__ sblock, const uint32_t* __restrict__ n, uint32_t nblock,
                  uint32_t* __restrict__ owner) {
-  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n) owner[sblock[i]] = sblock[headpos[i]];  // headpos: inclusive max-scan of the head positions
+  const uint32_t lane = threadIdx.x & 31u;
+  const uint64_t i = (blockIdx.x * (uint64_t)blockDim.x + threadIdx.x) >> 5;
+  if (i >= nblock) return;
+  const uint32_t b = sblock[i];
+  uint32_t o = b;
+  for (uint32_t j = headpos[i]; j < i; j++) {
+    const uint32_t c = sblock[j];
+    if (n[c] == n[b] && cs_same_table<T, CS_PER_LANE>(in, d, c, b, lane)) {
+      o = c;
+      break;
+    }
+  }
+  if (lane == 0) owner[b] = o;
 }
 
 template <int WORDS>
@@ -167,16 +227,23 @@ __global__ void __launch_bounds__(256)
   size[b] = (bits * bvox + 31) / 32 + (owner[b] == b ? n[b] * WORDS : 0u);
 }
 
-// offsets from the channel start: indices at 2*nblock + scan[b]; own tables right after them
+// offsets from the channel start: indices at 2*nblock + scan[b]; own tables right after them.
+// *max_toff = the largest table offset (the format stores it in 24 bits).
 __global__ void __launch_bounds__(256)
     k_cseg_offsets(const uint32_t* __restrict__ n, const uint32_t* __restrict__ owner, const uint32_t* __restrict__ scan,
-                   uint32_t nblock, uint32_t bvox, uint32_t* __restrict__ enc_off, uint32_t* __restrict__ tab_off) {
+                   uint32_t nblock, uint32_t bvox, uint32_t* __restrict__ enc_off, uint32_t* __restrict__ tab_off,
+                   uint32_t* __restrict__ max_toff) {
   const uint32_t b = blockIdx.x * blockDim.x + threadIdx.x;
-  if (b >= nblock) return;
-  enc_off[b] = 2 * nblock + scan[b];
-  const uint32_t o = owner[b];
-  const uint32_t obits = cs_bits(n[o]);
-  tab_off[b] = 2 * nblock + scan[o] + (obits * bvox + 31) / 32;
+  uint32_t t = 0;
+  if (b < nblock) {
+    enc_off[b] = 2 * nblock + scan[b];
+    const uint32_t o = owner[b];
+    const uint32_t obits = cs_bits(n[o]);
+    t = 2 * nblock + scan[o] + (obits * bvox + 31) / 32;
+    tab_off[b] = t;
+  }
+  t = __reduce_max_sync(CS_FULL, t);
+  if ((threadIdx.x & 31u) == 0 && t != 0) atomicMax(max_toff, t);
 }
 
 template <typename T>
@@ -239,7 +306,7 @@ static int cseg_encode_channel(ign_ctx* ctx, const T* in, const CsegDims& d, uin
     if (mb > scanb) scanb = mb;
   }
   const size_t tmpb = (sortb > scanb ? sortb : scanb) + 256;
-  if (own) IGN_TRY(scratch_reserve(ctx, 2 * align_up((size_t)nb * 8, 256) + 8 * align_up(((size_t)nb + 1) * 4, 256) + tmpb + 4096));
+  if (own) IGN_TRY(scratch_reserve(ctx, 2 * align_up((size_t)nb * 8, 256) + 8 * align_up(((size_t)nb + 2) * 4, 256) + tmpb + 4096));
   auto fail = [&](int rc) {
     ctx->scratch_used = keep;
     return rc;
@@ -251,7 +318,7 @@ static int cseg_encode_channel(ign_ctx* ctx, const T* in, const CsegDims& d, uin
   uint32_t* sblk = (uint32_t*)scratch_take(ctx, ((size_t)nb + 1) * 4);
   uint32_t* owner = (uint32_t*)scratch_take(ctx, ((size_t)nb + 1) * 4);
   uint32_t* size = (uint32_t*)scratch_take(ctx, ((size_t)nb + 1) * 4);
-  uint32_t* scan = (uint32_t*)scratch_take(ctx, ((size_t)nb + 1) * 4);
+  uint32_t* scan = (uint32_t*)scratch_take(ctx, ((size_t)nb + 2) * 4);  // [nb]: total, [nb + 1]: largest table offset
   uint32_t* enc_off = (uint32_t*)scratch_take(ctx, ((size_t)nb + 1) * 4);
   uint32_t* tab_off = (uint32_t*)scratch_take(ctx, ((size_t)nb + 1) * 4);
   void* tmp = scratch_take(ctx, tmpb);
@@ -292,7 +359,10 @@ static int cseg_encode_channel(ign_ctx* ctx, const T* in, const CsegDims& d, uin
     CS_CUDA(cub::DeviceScan::InclusiveScan(tmp, tb, enc_off, tab_off, cub::Max(), (int)nb, ctx->stream));
     ctx->launches += 2;
   }
-  CS_LAUNCH(k_cseg_owner, blocks_for(nb, 256), 256, tab_off, sblk, nb, owner);
+  if (d.bvox <= 512)
+    CS_LAUNCH((k_cseg_owner<T, 16>), gw, 128, in, d, tab_off, sblk, n, nb, owner);
+  else
+    CS_LAUNCH((k_cseg_owner<T, 32>), gw, 128, in, d, tab_off, sblk, n, nb, owner);
   CS_LAUNCH((k_cseg_sizes<WORDS>), blocks_for(nb, 256), 256, n, owner, nb, d.bvox, size);
   CS_CUDA(cudaMemsetAsync(size + nb, 0, 4, ctx->stream));
   {
@@ -300,21 +370,23 @@ static int cseg_encode_channel(ign_ctx* ctx, const T* in, const CsegDims& d, uin
     CS_CUDA(cub::DeviceScan::ExclusiveSum(tmp, tb, size, scan, (int)nb + 1, ctx->stream));
     ctx->launches += 2;
   }
-  uint32_t total = 0;
+  CS_CUDA(cudaMemsetAsync(scan + nb + 1, 0, 4, ctx->stream));
+  CS_LAUNCH(k_cseg_offsets, blocks_for(nb, 256), 256, n, owner, scan, nb, d.bvox, enc_off, tab_off, scan + nb + 1);
+  uint32_t tail[2] = {0, 0};  // words after the headers, largest table offset
   {
-    const int rc = small_d2h(ctx, &total, scan + nb, 4);
+    const int rc = small_d2h(ctx, tail, scan + nb, 8);
     if (rc != IGN_OK) return fail(rc);
     const int rc2 = small_sync(ctx);
     if (rc2 != IGN_OK) return fail(rc2);
   }
-  const uint64_t words = 2ull * nb + total;
+  const uint64_t words = 2ull * nb + tail[0];
   *n_words = words;
-  if (words > 0xFFFFFFull + 1024) {
-    set_error("cseg: the encoded chunk (%llu words) exceeds the format's 24-bit table offsets", (unsigned long long)words);
+  if (tail[1] > 0xFFFFFFu) {
+    set_error("cseg: a lookup table of the encoded chunk starts at word %u, beyond the format's 24-bit table offsets",
+              tail[1]);
     return fail(IGN_ERR_OVERFLOW);
   }
   if (out_dev != nullptr && words <= cap_words) {
-    CS_LAUNCH(k_cseg_offsets, blocks_for(nb, 256), 256, n, owner, scan, nb, d.bvox, enc_off, tab_off);
     if (d.bvox <= 512)
       CS_LAUNCH((k_cseg_scan<T, true, 16>), gw, 128, in, d, (uint64_t)nb, (uint32_t*)nullptr, (unsigned long long*)nullptr,
                 enc_off, tab_off, owner, out_dev);

@@ -18,9 +18,13 @@ constexpr uint64_t HT_EMPTY = ~0ull;
 constexpr uint32_t HT_NONE = 0xFFFFFFFFu;
 constexpr unsigned FULLM = 0xFFFFFFFFu;
 
+// The key HT_EMPTY (2^64-1) marks a free slot, so it cannot be stored in keys[]; it gets a
+// side slot instead: index mask + 1, present when *side != 0, payload vals[mask + 1].  Every
+// lookup of that key goes through the side slot, so all 2^64 labels are valid keys.
 struct HashTable {
   uint64_t* keys;  // [cap]
-  uint64_t* vals;  // [cap] payload (first index / count / mapped value)
+  uint64_t* vals;  // [cap + 1] payload (first index / count / mapped value)
+  uint32_t* side;  // present flag of the key HT_EMPTY
   uint32_t mask;   // cap - 1
 };
 
@@ -28,8 +32,20 @@ __device__ __forceinline__ uint32_t ht_hash(uint64_t key, uint32_t mask) {
   return (uint32_t)(mix64(key) >> 17) & mask;
 }
 
+// key stored in slot s (s <= mask + 1); only meaningful for an occupied slot
+__device__ __forceinline__ uint64_t ht_key(const HashTable& t, uint32_t s) {
+  return s > t.mask ? HT_EMPTY : t.keys[s];
+}
+__device__ __forceinline__ bool ht_occupied(const HashTable& t, uint32_t s) {
+  return s <= t.mask ? t.keys[s] != HT_EMPTY : (s == t.mask + 1 && *t.side != 0);
+}
+
 // returns slot of key, inserting it if absent; HT_NONE when the table is full
 __device__ __forceinline__ uint32_t ht_insert(const HashTable& t, uint64_t key, uint32_t* counters) {
+  if (key == HT_EMPTY) {
+    if (((volatile uint32_t*)t.side)[0] == 0 && atomicExch(t.side, 1u) == 0) atomicAdd(&counters[0], 1u);
+    return t.mask + 1;
+  }
   uint32_t h = ht_hash(key, t.mask);
   for (uint32_t probes = 0; probes <= t.mask; probes++) {
     const uint64_t cur = ((volatile uint64_t*)t.keys)[h];
@@ -50,6 +66,7 @@ __device__ __forceinline__ uint32_t ht_insert(const HashTable& t, uint64_t key, 
 }
 
 __device__ __forceinline__ uint32_t ht_find(const HashTable& t, uint64_t key) {
+  if (key == HT_EMPTY) return *t.side ? t.mask + 1 : HT_NONE;
   uint32_t h = ht_hash(key, t.mask);
   for (uint32_t probes = 0; probes <= t.mask; probes++) {
     const uint64_t cur = t.keys[h];
@@ -73,21 +90,17 @@ __global__ void __launch_bounds__(256)
   if (i >= n) return;
   const T v = in[i];
   if (i > 0 && in[i - 1] == v) return;
-  if ((uint64_t)v == HT_EMPTY) {
-    counters[2] = 1;  // reserved key
-    return;
-  }
   const uint32_t h = ht_insert(t, (uint64_t)v, counters);
   if (h != HT_NONE) atomicMin((unsigned long long*)&t.vals[h], (unsigned long long)i);
 }
 
-// occupied slots -> (first index, slot) lists
+// occupied slots (side slot included: launch over cap + 1 threads) -> (first index, slot) lists
 __global__ void __launch_bounds__(256)
     k_compact_slots(HashTable t, uint64_t* __restrict__ firsts, uint32_t* __restrict__ slots,
                     uint32_t* counters) {
   const uint32_t s = blockIdx.x * blockDim.x + threadIdx.x;
   const uint32_t lane = threadIdx.x & 31;
-  const bool occ = (s <= t.mask) && (t.keys[s] != HT_EMPTY);
+  const bool occ = ht_occupied(t, s);
   const uint32_t m = __ballot_sync(FULLM, occ);
   if (m) {
     const int leader = __ffs(m) - 1;
@@ -106,7 +119,7 @@ __global__ void __launch_bounds__(256)
     k_find_zero(HashTable t, const uint32_t* __restrict__ slots_sorted, uint32_t k,
                 uint32_t* counters) {
   const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
-  if (j < k && t.keys[slots_sorted[j]] == 0) counters[4] = j;
+  if (j < k && ht_key(t, slots_sorted[j]) == 0) counters[4] = j;
 }
 
 __global__ void __launch_bounds__(256)
@@ -117,7 +130,7 @@ __global__ void __launch_bounds__(256)
   if (j >= k) return;
   const uint32_t zero_pos = counters[4];
   const uint32_t s = slots_sorted[j];
-  const uint64_t key = t.keys[s];
+  const uint64_t key = ht_key(t, s);
   uint64_t id = 0;
   if (key != 0) {
     id = (uint64_t)j + 1 - ((zero_pos != HT_NONE && j > zero_pos) ? 1 : 0);
@@ -182,10 +195,6 @@ __global__ void __launch_bounds__(256)
   const bool head = inb && (lane == 0 || vl != vv);
   const uint32_t hm = __ballot_sync(FULLM, head || !inb);
   if (head) {
-    if ((uint64_t)v == HT_EMPTY) {
-      counters[2] = 1;
-      return;
-    }
     const uint32_t above = (lane == 31) ? 0u : (hm & ~((2u << lane) - 1u));
     const uint32_t end = above ? (uint32_t)(__ffs(above) - 1) : 32u;
     const uint32_t h = ht_insert(t, (uint64_t)v, counters);
@@ -198,7 +207,7 @@ __global__ void __launch_bounds__(256)
                  uint32_t* counters) {
   const uint32_t s = blockIdx.x * blockDim.x + threadIdx.x;
   const uint32_t lane = threadIdx.x & 31;
-  const bool occ = (s <= t.mask) && (t.keys[s] != HT_EMPTY);
+  const bool occ = ht_occupied(t, s);
   const uint32_t m = __ballot_sync(FULLM, occ);
   if (m) {
     const int leader = __ffs(m) - 1;
@@ -207,7 +216,7 @@ __global__ void __launch_bounds__(256)
     base = __shfl_sync(FULLM, base, leader);
     if (occ) {
       const uint32_t pos = base + __popc(m & ((1u << lane) - 1u));
-      keys[pos] = t.keys[s];
+      keys[pos] = ht_key(t, s);
       vals[pos] = t.vals[s];
     }
   }
@@ -260,12 +269,13 @@ static uint32_t pow2_at_least(uint64_t v) {
 static int table_alloc(ign_ctx* ctx, uint32_t cap, uint64_t val_init_byte, HashTable& t,
                        uint32_t** counters) {
   t.keys = (uint64_t*)scratch_take(ctx, (size_t)cap * 8);
-  t.vals = (uint64_t*)scratch_take(ctx, (size_t)cap * 8);
+  t.vals = (uint64_t*)scratch_take(ctx, ((size_t)cap + 1) * 8);
   *counters = (uint32_t*)scratch_take(ctx, 256);
   IGN_REQUIRE(t.keys && t.vals && *counters, IGN_ERR_NOMEM, "scratch arena too small for hash table");
+  t.side = *counters + 2;
   t.mask = cap - 1;
   IGN_CUDA(cudaMemsetAsync(t.keys, 0xFF, (size_t)cap * 8, ctx->stream));
-  IGN_CUDA(cudaMemsetAsync(t.vals, (int)val_init_byte, (size_t)cap * 8, ctx->stream));
+  IGN_CUDA(cudaMemsetAsync(t.vals, (int)val_init_byte, ((size_t)cap + 1) * 8, ctx->stream));
   IGN_CUDA(cudaMemsetAsync(*counters, 0, 256, ctx->stream));
   IGN_CUDA(cudaMemsetAsync(*counters + 4, 0xFF, 4, ctx->stream));  // zero_pos = NONE
   return IGN_OK;
@@ -315,7 +325,6 @@ static int renumber_table(ign_ctx* ctx, const void* in, int dtype, uint64_t n, H
 #undef RUN_FIRST
     uint32_t h[8];
     IGN_TRY(read_counters(ctx, counters, h));
-    IGN_REQUIRE(h[2] == 0, IGN_ERR_UNSUPPORTED, "label 2^64-1 is reserved by the hash table");
     if (h[1] != 0 || h[0] > cap / 2) {
       IGN_REQUIRE(cap < cap_max, IGN_ERR_OVERFLOW, "renumber: hash table overflow at maximum capacity");
       cap = (cap > cap_max / 8) ? cap_max : cap * 8;
@@ -331,7 +340,7 @@ static int renumber_table(ign_ctx* ctx, const void* in, int dtype, uint64_t n, H
     IGN_REQUIRE(firsts && slots && firsts_s && slots_s && tmp, IGN_ERR_NOMEM, "scratch arena too small (renumber)");
     uint64_t k = 0;
     if (total > 0) {
-      IGN_LAUNCH(ctx, k_compact_slots, blocks_for((uint64_t)cap, 256), 256, 0, t, firsts, slots, counters);
+      IGN_LAUNCH(ctx, k_compact_slots, blocks_for((uint64_t)cap + 1, 256), 256, 0, t, firsts, slots, counters);
       int end_bit = 1;
       while (end_bit < 64 && (1ull << end_bit) < n) end_bit++;
       IGN_CUDA(cub::DeviceRadixSort::SortPairs(tmp, tmp_bytes, firsts, firsts_s, slots, slots_s,
@@ -537,7 +546,6 @@ int ign_unique(ign_ctx* ctx, const void* in, int dtype, uint64_t n, uint64_t* un
 #undef RUN_COUNT
     uint32_t h[8];
     IGN_TRY(read_counters(ctx, counters, h));
-    IGN_REQUIRE(h[2] == 0, IGN_ERR_UNSUPPORTED, "label 2^64-1 is reserved by the hash table");
     if (h[1] != 0 || h[0] > cap / 2) {
       IGN_REQUIRE(cap < cap_max, IGN_ERR_OVERFLOW, "unique: hash table overflow");
       cap = (cap > cap_max / 8) ? cap_max : cap * 8;
@@ -553,7 +561,7 @@ int ign_unique(ign_ctx* ctx, const void* in, int dtype, uint64_t n, uint64_t* un
       size_t tmp_bytes = sort_tmp_bytes_u64(total);
       void* tmp = scratch_take(ctx, tmp_bytes);
       IGN_REQUIRE(ck && cv && sk && sv && tmp, IGN_ERR_NOMEM, "scratch arena too small (unique)");
-      IGN_LAUNCH(ctx, k_compact_kv, blocks_for((uint64_t)cap, 256), 256, 0, t, ck, cv, counters);
+      IGN_LAUNCH(ctx, k_compact_kv, blocks_for((uint64_t)cap + 1, 256), 256, 0, t, ck, cv, counters);
       IGN_CUDA(cub::DeviceRadixSort::SortPairs(tmp, tmp_bytes, ck, sk, cv, sv, (int)total, 0, 64, ctx->stream));
       ctx->launches += 2;
       const uint64_t m = total < capacity ? total : capacity;

@@ -277,7 +277,8 @@ IGN_API int ign_mesh_free(ign_mesher* m);
  * output, igneous/task_creation/common.py:215-236 set_encoding).  labels: Fortran order [x,y,z,c],
  * uint32 / uint64; block (bx,by,bz) is (8,8,8) in every Precomputed layer.  The stream is the
  * uint32 word sequence of the file.  encode: *n_words = words needed; nothing is written when
- * out is NULL or cap_words is too small.  One call = one chunk (24-bit table offsets). */
+ * out is NULL or cap_words is too small.  One call = one chunk: IGN_ERR_OVERFLOW when a lookup table
+ * of a channel would start at word 2^24 or later (the header stores table offsets in 24 bits). */
 IGN_API int ign_cseg_encode(ign_ctx* ctx, const void* labels, int dtype, uint64_t sx, uint64_t sy, uint64_t sz,
                             uint64_t sc, uint32_t bx, uint32_t by, uint32_t bz, uint32_t* out,
                             uint64_t cap_words, uint64_t* n_words);
