@@ -48,6 +48,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <memory>
 #include <type_traits>
 #include <vector>
 
@@ -987,7 +988,7 @@ static uint64_t default_rcap(uint64_t n) { return n / 8 + 4096; }
 // of every run and plan.ncomp is on the host.  `rcap` = run capacity reserved in the arena;
 // *need_rcap > rcap on return means the volume has more runs (nothing else is valid).
 template <typename R>
-static int ccl_structure(ign_ctx* ctx, const R& rd, uint32_t sx, uint32_t sy, uint32_t sz, uint64_t rcap,
+static int ccl_structure(ign_ctx* ctx, Scratch& sc, const R& rd, uint32_t sx, uint32_t sy, uint32_t sz, uint64_t rcap,
                          CclPlan& p, uint64_t* need_rcap) {
   using T = typename R::value_type;
   using MT = MaskTile<T>;
@@ -998,18 +999,17 @@ static int ccl_structure(ign_ctx* ctx, const R& rd, uint32_t sx, uint32_t sy, ui
   p.R = 0;
   p.ncomp = 0;
   const uint64_t W = p.W;
-  p.S = (uint32_t*)scratch_take(ctx, (W + 2) * 4);
-  p.Z = (uint32_t*)scratch_take(ctx, (W + 2) * 4);
-  p.Ey = (uint32_t*)scratch_take(ctx, (W + 2) * 4);
-  p.Ez = (uint32_t*)scratch_take(ctx, (W + 2) * 4);
-  p.rbase = (uint32_t*)scratch_take(ctx, (W + 2) * 4);
-  p.label = (uint32_t*)scratch_take(ctx, (rcap + 2) * 4);
-  p.rank = (uint32_t*)scratch_take(ctx, (rcap + 2) * 4);
+  p.S = sc.take<uint32_t>(W + 2);
+  p.Z = sc.take<uint32_t>(W + 2);
+  p.Ey = sc.take<uint32_t>(W + 2);
+  p.Ez = sc.take<uint32_t>(W + 2);
+  p.rbase = sc.take<uint32_t>(W + 2);
+  p.label = sc.take<uint32_t>(rcap + 2);
+  p.rank = sc.take<uint32_t>(rcap + 2);
   const uint64_t items = (W + 1 > rcap + 1 ? W + 1 : rcap + 1);
   p.cub_bytes = ccl_cub_bytes(items);
-  p.cub_tmp = scratch_take(ctx, p.cub_bytes);
-  IGN_REQUIRE(p.S && p.Z && p.Ey && p.Ez && p.rbase && p.label && p.rank && p.cub_tmp, IGN_ERR_NOMEM,
-              "CCL scratch arena too small");
+  p.cub_tmp = sc.take(p.cub_bytes);
+  IGN_REQUIRE(sc.ok(), IGN_ERR_NOMEM, "CCL scratch arena too small");
   *need_rcap = 0;
 
   // ---- pass A
@@ -1178,19 +1178,19 @@ static int launch_expand(ign_ctx* ctx, const CclPlan& p, uint64_t offset, void* 
 
 // dust on the run labels of p: components with fewer than `threshold` voxels get label 0,
 // the others are renumbered 1..kept in the same order.
-static int dust_runs(ign_ctx* ctx, CclPlan& p, uint64_t threshold, uint32_t* kept) {
+static int dust_runs(ign_ctx* ctx, Scratch& sc, CclPlan& p, uint64_t threshold, uint32_t* kept) {
   const uint32_t N = p.ncomp;
   *kept = N;
   if (N == 0 || p.R == 0) return IGN_OK;
   const size_t bytes = ((size_t)N + 2) * 4;
-  uint32_t* counts = (uint32_t*)scratch_take(ctx, bytes);
-  uint32_t* keep = (uint32_t*)scratch_take(ctx, bytes);
-  uint32_t* scan = (uint32_t*)scratch_take(ctx, bytes);
-  uint32_t* lut = (uint32_t*)scratch_take(ctx, bytes);
+  uint32_t* counts = sc.take<uint32_t>((size_t)N + 2);
+  uint32_t* keep = sc.take<uint32_t>((size_t)N + 2);
+  uint32_t* scan = sc.take<uint32_t>((size_t)N + 2);
+  uint32_t* lut = sc.take<uint32_t>((size_t)N + 2);
   size_t tb = 0;
   cub::DeviceScan::ExclusiveSum(nullptr, tb, (const uint32_t*)nullptr, (uint32_t*)nullptr, (int)(N + 2));
-  void* tmp = scratch_take(ctx, tb + 256);
-  IGN_REQUIRE(counts && keep && scan && lut && tmp, IGN_ERR_NOMEM, "scratch arena too small for dust maps");
+  void* tmp = sc.take(tb + 256);
+  IGN_REQUIRE(sc.ok(), IGN_ERR_NOMEM, "scratch arena too small for dust maps");
   IGN_CUDA(cudaMemsetAsync(counts, 0, bytes, ctx->stream));
   const ExpandArgs e = p.expand_args(0);
   IGN_LAUNCH(ctx, k_ccl_count, blocks_for(p.W, 256), 256, 0, e, counts);
@@ -1213,51 +1213,30 @@ static int ccl_run(ign_ctx* ctx, const R& rd, uint64_t sx, uint64_t sy, uint64_t
                    TL* dust_labels_inplace, uint64_t* n_components) {
   IGN_TRY(check_ccl_dims(sx, sy, sz));
   const uint64_t n = sx * sy * sz, W = ((sx + 31) / 32) * sy * sz;
-  const bool own_arena = (ctx->scratch_used == 0);
+  Scratch sc(ctx);
   uint64_t rcap = default_rcap(n);
   for (int attempt = 0; attempt < 2; attempt++) {
-    const size_t keep_used = ctx->scratch_used;
-    auto fail = [&](int rc) {
-      ctx->scratch_used = keep_used;
-      return rc;
-    };
-    if (own_arena) {
-      const int rc = scratch_reserve(ctx, ccl_scratch_bytes(W, rcap) + 6 * (rcap + 4) * 4 + 65536);
-      if (rc != IGN_OK) return fail(rc);
-    }
+    sc.rewind();
+    IGN_TRY(sc.reserve(ccl_scratch_bytes(W, rcap) + 6 * (rcap + 4) * 4 + 65536));
     CclPlan p;
     uint64_t need = 0;
-    int rc = ccl_structure(ctx, rd, (uint32_t)sx, (uint32_t)sy, (uint32_t)sz, rcap, p, &need);
-    if (rc != IGN_OK) return fail(rc);
+    IGN_TRY(ccl_structure(ctx, sc, rd, (uint32_t)sx, (uint32_t)sy, (uint32_t)sz, rcap, p, &need));
     if (need > rcap) {
-      ctx->scratch_used = keep_used;
       IGN_REQUIRE(attempt == 0, IGN_ERR_NOMEM, "CCL: %llu runs do not fit the scratch arena", (unsigned long long)need);
       rcap = need + 16;
       continue;
     }
     uint32_t kept = p.ncomp;
-    if (dust_threshold > 0 && p.ncomp > 0) {
-      rc = dust_runs(ctx, p, dust_threshold, &kept);
-      if (rc != IGN_OK) return fail(rc);
-    }
+    if (dust_threshold > 0 && p.ncomp > 0) IGN_TRY(dust_runs(ctx, sc, p, dust_threshold, &kept));
     if (dust_labels_inplace != nullptr && dust_threshold > 0 && p.R > 0) {
       const ExpandArgs e = p.expand_args(0);
       IGN_LAUNCH(ctx, (k_dust_apply<TL>), blocks_for(p.W * 32, 256), 256, 0, e, dust_labels_inplace);
     }
     if (out != nullptr) {
-      if (p.R == 0) {
-        cudaError_t e = cudaMemsetAsync(out, 0, n * dtype_size(out_dtype), ctx->stream);
-        if (e != cudaSuccess) {
-          set_error("CCL: memset failed: %s", cudaGetErrorString(e));
-          return fail(IGN_ERR_CUDA);
-        }
-      } else {
-        rc = launch_expand(ctx, p, offset, out, out_dtype, kept);
-        if (rc != IGN_OK) return fail(rc);
-      }
+      if (p.R == 0) IGN_CUDA(cudaMemsetAsync(out, 0, n * dtype_size(out_dtype), ctx->stream));
+      else IGN_TRY(launch_expand(ctx, p, offset, out, out_dtype, kept));
     }
     if (n_components) *n_components = kept;
-    ctx->scratch_used = keep_used;
     return IGN_OK;
   }
   return IGN_ERR_OVERFLOW;
@@ -1306,19 +1285,20 @@ struct ign_ccl_volume {
   int in_dtype;
   CclPlan plan;
   uint64_t n_local;
+  size_t base;  // the masks and run labels are held in the arena above this
 };
 
 template <typename T>
-static int volume_begin_typed(ign_ctx* ctx, ign_ccl_volume* v, uint64_t sx, uint64_t sy, uint64_t sz,
+static int volume_begin_typed(ign_ctx* ctx, Scratch& sc, ign_ccl_volume* v, uint64_t sx, uint64_t sy, uint64_t sz,
                               uint64_t* first_values, uint32_t* first_labels, uint64_t* last_values,
                               uint32_t* last_labels) {
   const uint64_t n = sx * sy * sz, W = ((sx + 31) / 32) * sy * sz;
   uint64_t rcap = default_rcap(n);
   for (int attempt = 0; attempt < 2; attempt++) {
-    scratch_reset(ctx);
-    IGN_TRY(scratch_reserve(ctx, ccl_scratch_bytes(W, rcap) + (rcap + 64) * 4 + 65536));
+    sc.rewind();
+    IGN_TRY(sc.reserve(ccl_scratch_bytes(W, rcap) + (rcap + 64) * 4 + 65536));
     uint64_t need = 0;
-    IGN_TRY(ccl_structure(ctx, plain_reader<T>(v->in), (uint32_t)sx, (uint32_t)sy, (uint32_t)sz, rcap, v->plan, &need));
+    IGN_TRY(ccl_structure(ctx, sc, plain_reader<T>(v->in), (uint32_t)sx, (uint32_t)sy, (uint32_t)sz, rcap, v->plan, &need));
     if (need > rcap) {
       IGN_REQUIRE(attempt == 0, IGN_ERR_NOMEM, "CCL: %llu runs do not fit the scratch arena", (unsigned long long)need);
       rcap = need + 16;
@@ -1344,39 +1324,23 @@ static int volume_begin_typed(ign_ctx* ctx, ign_ccl_volume* v, uint64_t sx, uint
   return IGN_OK;
 }
 
-static int grow(char** buf, size_t* have, size_t need) {
-  if (*have >= need) return IGN_OK;
-  if (*buf) cudaFree(*buf);
-  *buf = nullptr;
-  *have = 0;
-  const size_t want = need + need / 4;
-  cudaError_t e = cudaMalloc((void**)buf, want);
-  if (e != cudaSuccess) {
-    cudaGetLastError();
-    set_error("multi-GPU CCL: cudaMalloc(%zu) failed: %s", want, cudaGetErrorString(e));
-    return IGN_ERR_NOMEM;
-  }
-  *have = want;
-  return IGN_OK;
-}
-
 // One rank's share of a CCL over a dataset that is split into z-slabs (rank r above rank r-1).
 // Exactly ONE collective: an all-gather of [n_local | first plane | last plane]; linking the
 // N-1 boundaries, the replicated union-find and the relabelling all run on the device.
 template <typename T>
-static int ccl_sharded_typed(ign_group* g, ign_ccl_volume* v, uint64_t sx, uint64_t sy, uint64_t sz, void* out,
+static int ccl_sharded_typed(ign_group* g, Scratch& sc, ign_ccl_volume* v, uint64_t sx, uint64_t sy, uint64_t sz, void* out,
                              int out_dtype, uint64_t* n_global) {
   ign_ctx* ctx = g->ctx;
   const int N = g->nranks, me = g->rank;
   const uint64_t np = sx * sy;
   const size_t rec = 256 + 2 * np * 8 + 2 * np * 4;
-  IGN_TRY(grow(&g->d_send, &g->send_bytes, rec));
-  IGN_TRY(grow(&g->d_recv, &g->recv_bytes, rec * (size_t)N));
+  IGN_TRY(grow_buffer(ctx, &g->d_send, &g->send_bytes, rec, "multi-GPU CCL"));
+  IGN_TRY(grow_buffer(ctx, &g->d_recv, &g->recv_bytes, rec * (size_t)N, "multi-GPU CCL"));
   uint64_t* first_v = (uint64_t*)(g->d_send + 256);
   uint64_t* last_v = first_v + np;
   uint32_t* first_l = (uint32_t*)(last_v + np);
   uint32_t* last_l = first_l + np;
-  IGN_TRY(volume_begin_typed<T>(ctx, v, sx, sy, sz, first_v, first_l, last_v, last_l));
+  IGN_TRY(volume_begin_typed<T>(ctx, sc, v, sx, sy, sz, first_v, first_l, last_v, last_l));
   CclPlan& p = v->plan;
   uint64_t head[32] = {0};
   head[0] = v->n_local;
@@ -1391,7 +1355,8 @@ static int ccl_sharded_typed(ign_group* g, ign_ccl_volume* v, uint64_t sx, uint6
   IGN_REQUIRE(total < 0x7FFFFFF0ull, IGN_ERR_OVERFLOW, "multi-GPU CCL: too many provisional components");
   const uint32_t items = (uint32_t)total + 2;  // ids 0..total and one sentinel
   const size_t cubb = ccl_cub_bytes(items);
-  IGN_TRY(grow(&g->d_solve, &g->solve_bytes, 2 * align_up((size_t)items * 4, 256) + align_up(cubb, 256)));
+  IGN_TRY(grow_buffer(ctx, &g->d_solve, &g->solve_bytes, 2 * align_up((size_t)items * 4, 256) + align_up(cubb, 256),
+                      "multi-GPU CCL"));
   uint32_t* parent = (uint32_t*)g->d_solve;
   uint32_t* rank = (uint32_t*)(g->d_solve + align_up((size_t)items * 4, 256));
   void* tmp = g->d_solve + 2 * align_up((size_t)items * 4, 256);
@@ -1488,24 +1453,15 @@ int ign_ccl6(ign_ctx* ctx, const void* in, int in_dtype, uint64_t sx, uint64_t s
   IGN_TRY(check_ccl_dims(sx, sy, sz));
   const int es = dtype_size(in_dtype), os = dtype_size(out_dtype);
   IGN_REQUIRE(es > 0 && os > 0, IGN_ERR_UNSUPPORTED, "unsupported dtype");
-  const uint64_t n = sx * sy * sz, W = ((sx + 31) / 32) * sy * sz;
-  scratch_reset(ctx);
-  const uint64_t rcap = n + 16;  // host path: size for the worst case once
-  IGN_TRY(scratch_reserve(ctx, align_up(n * es, 256) + align_up(n * os, 256) + ccl_scratch_bytes(W, rcap) + 6 * (rcap + 4) * 4 + 65536));
-  void* d_in = scratch_take(ctx, n * es);
-  void* d_out = scratch_take(ctx, n * os);
-  IGN_CUDA(cudaMemcpyAsync(d_in, in, n * es, cudaMemcpyHostToDevice, ctx->stream));
-  int rc = ign_ccl6_dev(ctx, d_in, in_dtype, sx, sy, sz, d_out, out_dtype, n_components);
-  if (rc == IGN_OK) {
-    cudaError_t e = cudaMemcpyAsync(out, d_out, n * os, cudaMemcpyDeviceToHost, ctx->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-    if (e != cudaSuccess) {
-      set_error("CCL D2H: %s", cudaGetErrorString(e));
-      rc = IGN_ERR_CUDA;
-    }
-  }
-  scratch_reset(ctx);
-  return rc;
+  const uint64_t n = sx * sy * sz;
+  Staging st(ctx);
+  void *d_in, *d_out;
+  st.add(&d_in, n * es, in);
+  st.add(&d_out, n * os);
+  IGN_TRY(st.stage());
+  IGN_TRY(ign_ccl6_dev(ctx, d_in, in_dtype, sx, sy, sz, d_out, out_dtype, n_components));
+  IGN_TRY(st.back(out, d_out, n * os));
+  return st.sync();
 }
 
 int ign_dust(ign_ctx* ctx, void* labels, int dtype, uint64_t sx, uint64_t sy, uint64_t sz,
@@ -1516,23 +1472,14 @@ int ign_dust(ign_ctx* ctx, void* labels, int dtype, uint64_t sx, uint64_t sy, ui
   IGN_TRY(check_ccl_dims(sx, sy, sz));
   const int es = dtype_size(dtype);
   IGN_REQUIRE(es > 0 && dtype != IGN_F32, IGN_ERR_UNSUPPORTED, "unsupported dtype");
-  const uint64_t n = sx * sy * sz, W = ((sx + 31) / 32) * sy * sz;
-  scratch_reset(ctx);
-  const uint64_t rcap = n + 16;
-  IGN_TRY(scratch_reserve(ctx, align_up(n * es, 256) + ccl_scratch_bytes(W, rcap) + 6 * (rcap + 4) * 4 + 65536));
-  void* d = scratch_take(ctx, n * es);
-  IGN_CUDA(cudaMemcpyAsync(d, labels, n * es, cudaMemcpyHostToDevice, ctx->stream));
-  int rc = ign_dust_dev(ctx, d, dtype, sx, sy, sz, threshold);
-  if (rc == IGN_OK) {
-    cudaError_t e = cudaMemcpyAsync(labels, d, n * es, cudaMemcpyDeviceToHost, ctx->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-    if (e != cudaSuccess) {
-      set_error("dust D2H: %s", cudaGetErrorString(e));
-      rc = IGN_ERR_CUDA;
-    }
-  }
-  scratch_reset(ctx);
-  return rc;
+  const uint64_t n = sx * sy * sz;
+  Staging st(ctx);
+  void* d;
+  st.add(&d, n * es, labels);
+  IGN_TRY(st.stage());
+  IGN_TRY(ign_dust_dev(ctx, d, dtype, sx, sy, sz, threshold));
+  IGN_TRY(st.back(labels, d, n * es));
+  return st.sync();
 }
 
 int ign_ccl6_link_dev(ign_ctx* ctx, const uint64_t* values_a, const uint32_t* labels_a,
@@ -1543,17 +1490,12 @@ int ign_ccl6_link_dev(ign_ctx* ctx, const uint64_t* values_a, const uint32_t* la
   IGN_REQUIRE(values_a && labels_a && values_b && labels_b && n_pairs, IGN_ERR_INVALID, "null argument");
   *n_pairs = 0;
   if (n_plane == 0) return IGN_OK;
-  const size_t keep = ctx->scratch_used;
-  const bool own = (keep == 0);
+  Scratch sc(ctx);
   const uint32_t cap = (uint32_t)(n_plane < 0x7FFFFFFFull ? n_plane : 0x7FFFFFFFull);
-  if (own) IGN_TRY(scratch_reserve(ctx, (size_t)cap * 16 + 8192));
-  uint64_t* d_pairs = (uint64_t*)scratch_take(ctx, (size_t)cap * 16);
-  uint32_t* counters = (uint32_t*)scratch_take(ctx, 256);
-  if (!d_pairs || !counters) {
-    ctx->scratch_used = keep;
-    set_error("scratch arena too small (CCL link)");
-    return IGN_ERR_NOMEM;
-  }
+  IGN_TRY(sc.reserve((size_t)cap * 16 + 8192));
+  uint64_t* d_pairs = sc.take<uint64_t>(2 * (size_t)cap);
+  uint32_t* counters = sc.take<uint32_t>(64);
+  IGN_REQUIRE(sc.ok(), IGN_ERR_NOMEM, "scratch arena too small (CCL link)");
   IGN_CUDA(cudaMemsetAsync(counters, 0, 256, ctx->stream));
   IGN_LAUNCH(ctx, k_ccl_link, blocks_for(n_plane, 256), 256, 0, values_a, labels_a, offset_a, values_b,
              labels_b, offset_b, n_plane, d_pairs, cap, counters);
@@ -1566,7 +1508,6 @@ int ign_ccl6_link_dev(ign_ctx* ctx, const uint64_t* values_a, const uint32_t* la
     const uint64_t m = total < capacity ? total : capacity;
     IGN_CUDA(cudaMemcpy(pairs_host, d_pairs, m * 16, cudaMemcpyDeviceToHost));
   }
-  ctx->scratch_used = keep;
   return IGN_OK;
 }
 
@@ -1608,7 +1549,7 @@ int ign_ccl6_solve(const uint64_t* pairs, uint64_t n_pairs, uint64_t total, uint
 
 int ign_ccl6_volume_abort(ign_ccl_volume* v) {
   if (!v) return IGN_OK;
-  scratch_reset(v->ctx);
+  Scratch held(v->ctx, v->base);  // releases the volume's bytes on return
   delete v;
   return IGN_OK;
 }
@@ -1621,26 +1562,23 @@ int ign_ccl6_volume_begin_dev(ign_ctx* ctx, const void* in, int in_dtype, uint64
   IGN_REQUIRE(in && out && n_local, IGN_ERR_INVALID, "null argument");
   *out = nullptr;
   IGN_TRY(check_ccl_dims(sx, sy, sz));
-  IGN_REQUIRE(ctx->scratch_used == 0, IGN_ERR_INVALID, "volume CCL must own the scratch arena");
-  ign_ccl_volume* v = new ign_ccl_volume();
+  Scratch sc(ctx);
+  IGN_REQUIRE(sc.owner(), IGN_ERR_INVALID, "volume CCL must own the scratch arena");
+  std::unique_ptr<ign_ccl_volume> v(new ign_ccl_volume());
   v->ctx = ctx;
   v->in = in;
   v->in_dtype = in_dtype;
-  int rc;
   switch (in_dtype) {
-    case IGN_U8: rc = volume_begin_typed<uint8_t>(ctx, v, sx, sy, sz, first_values, first_labels, last_values, last_labels); break;
-    case IGN_U16: rc = volume_begin_typed<uint16_t>(ctx, v, sx, sy, sz, first_values, first_labels, last_values, last_labels); break;
-    case IGN_U32: rc = volume_begin_typed<uint32_t>(ctx, v, sx, sy, sz, first_values, first_labels, last_values, last_labels); break;
-    case IGN_U64: rc = volume_begin_typed<uint64_t>(ctx, v, sx, sy, sz, first_values, first_labels, last_values, last_labels); break;
-    default: set_error("volume CCL: unsupported input dtype %d", in_dtype); rc = IGN_ERR_UNSUPPORTED;
-  }
-  if (rc != IGN_OK) {
-    ign_ccl6_volume_abort(v);
-    return rc;
+    case IGN_U8: IGN_TRY(volume_begin_typed<uint8_t>(ctx, sc, v.get(), sx, sy, sz, first_values, first_labels, last_values, last_labels)); break;
+    case IGN_U16: IGN_TRY(volume_begin_typed<uint16_t>(ctx, sc, v.get(), sx, sy, sz, first_values, first_labels, last_values, last_labels)); break;
+    case IGN_U32: IGN_TRY(volume_begin_typed<uint32_t>(ctx, sc, v.get(), sx, sy, sz, first_values, first_labels, last_values, last_labels)); break;
+    case IGN_U64: IGN_TRY(volume_begin_typed<uint64_t>(ctx, sc, v.get(), sx, sy, sz, first_values, first_labels, last_values, last_labels)); break;
+    default: set_error("volume CCL: unsupported input dtype %d", in_dtype); return IGN_ERR_UNSUPPORTED;
   }
   // the arena stays held (the masks and run labels live in it) until finish / abort
+  v->base = sc.keep();
   *n_local = v->n_local;
-  *out = v;
+  *out = v.release();
   return IGN_OK;
 }
 
@@ -1651,50 +1589,24 @@ int ign_ccl6_volume_finish_dev(ign_ccl_volume* v, const uint32_t* global_lut, ui
   IGN_REQUIRE(v && out, IGN_ERR_INVALID, "null argument");
   ign_ctx* ctx = v->ctx;
   IGN_TRY(activate(ctx));
+  std::unique_ptr<ign_ccl_volume> done(v);
+  Scratch sc(ctx, v->base);  // releases the volume's bytes on return
   CclPlan& p = v->plan;
-  int rc = IGN_OK;
   if (!global_lut) max_label = v->n_local;
   if (p.R == 0) {
-    const uint64_t n = (uint64_t)p.sx * p.sy * p.sz;
-    if (dtype_size(out_dtype) <= 0) {
-      set_error("unsupported out dtype");
-      rc = IGN_ERR_UNSUPPORTED;
-    } else if (cudaMemsetAsync(out, 0, n * dtype_size(out_dtype), ctx->stream) != cudaSuccess) {
-      set_error("volume CCL: memset failed");
-      rc = IGN_ERR_CUDA;
-    }
-  } else {
-    if (global_lut) {
-      uint32_t* d_lut = (uint32_t*)scratch_take(ctx, (v->n_local + 1) * 4);
-      if (!d_lut) {
-        set_error("scratch arena too small for the relabel table (%llu components)", (unsigned long long)v->n_local);
-        rc = IGN_ERR_NOMEM;
-      } else {
-        cudaError_t e = cudaMemcpyAsync(d_lut, global_lut, (v->n_local + 1) * 4, cudaMemcpyHostToDevice, ctx->stream);
-        if (e != cudaSuccess) {
-          set_error("volume CCL: lut H2D: %s", cudaGetErrorString(e));
-          rc = IGN_ERR_CUDA;
-        }
-        if (rc == IGN_OK) {
-          k_ccl_relabel_runs<<<blocks_for(p.R, 256), 256, 0, ctx->stream>>>(p.label, p.R, d_lut);
-          ctx->launches++;
-          if (cudaGetLastError() != cudaSuccess) {
-            set_error("volume CCL: relabel launch failed");
-            rc = IGN_ERR_CUDA;
-          }
-        }
-        // the host table may be a temporary of the caller
-        if (rc == IGN_OK && cudaStreamSynchronize(ctx->stream) != cudaSuccess) {
-          set_error("volume CCL: sync failed");
-          rc = IGN_ERR_CUDA;
-        }
-      }
-    }
-    if (rc == IGN_OK) rc = launch_expand(ctx, p, 0, out, out_dtype, max_label);
+    IGN_REQUIRE(dtype_size(out_dtype) > 0, IGN_ERR_UNSUPPORTED, "unsupported out dtype");
+    IGN_CUDA(cudaMemsetAsync(out, 0, (uint64_t)p.sx * p.sy * p.sz * dtype_size(out_dtype), ctx->stream));
+    return IGN_OK;
   }
-  scratch_reset(ctx);
-  delete v;
-  return rc;
+  if (global_lut) {
+    uint32_t* d_lut = sc.take<uint32_t>(v->n_local + 1);
+    IGN_REQUIRE(sc.ok(), IGN_ERR_NOMEM, "scratch arena too small for the relabel table (%llu components)",
+                (unsigned long long)v->n_local);
+    IGN_CUDA(cudaMemcpyAsync(d_lut, global_lut, (v->n_local + 1) * 4, cudaMemcpyHostToDevice, ctx->stream));
+    IGN_LAUNCH(ctx, k_ccl_relabel_runs, blocks_for(p.R, 256), 256, 0, p.label, p.R, d_lut);
+    IGN_CUDA(cudaStreamSynchronize(ctx->stream));  // the host table may be a temporary of the caller
+  }
+  return launch_expand(ctx, p, 0, out, out_dtype, max_label);
 }
 
 int ign_ccl6_volume_dev(ign_ctx* ctx, const void* in, int in_dtype, uint64_t sx, uint64_t sy,
@@ -1716,21 +1628,20 @@ int ign_ccl6_sharded_dev(ign_group* g, const void* in, int in_dtype, uint64_t sx
   IGN_TRY(activate(ctx));
   IGN_TRY(check_ccl_dims(sx, sy, sz));
   IGN_REQUIRE(dtype_size(out_dtype) > 0, IGN_ERR_UNSUPPORTED, "unsupported out dtype");
-  IGN_REQUIRE(ctx->scratch_used == 0, IGN_ERR_INVALID, "sharded CCL must own the scratch arena");
+  Scratch sc(ctx);
+  IGN_REQUIRE(sc.owner(), IGN_ERR_INVALID, "sharded CCL must own the scratch arena");
   ign_ccl_volume v;
   v.ctx = ctx;
   v.in = in;
   v.in_dtype = in_dtype;
-  int rc;
   switch (in_dtype) {
-    case IGN_U8: rc = ccl_sharded_typed<uint8_t>(g, &v, sx, sy, sz, out, out_dtype, n_global); break;
-    case IGN_U16: rc = ccl_sharded_typed<uint16_t>(g, &v, sx, sy, sz, out, out_dtype, n_global); break;
-    case IGN_U32: rc = ccl_sharded_typed<uint32_t>(g, &v, sx, sy, sz, out, out_dtype, n_global); break;
-    case IGN_U64: rc = ccl_sharded_typed<uint64_t>(g, &v, sx, sy, sz, out, out_dtype, n_global); break;
-    default: set_error("sharded CCL: unsupported input dtype %d", in_dtype); rc = IGN_ERR_UNSUPPORTED;
+    case IGN_U8: return ccl_sharded_typed<uint8_t>(g, sc, &v, sx, sy, sz, out, out_dtype, n_global);
+    case IGN_U16: return ccl_sharded_typed<uint16_t>(g, sc, &v, sx, sy, sz, out, out_dtype, n_global);
+    case IGN_U32: return ccl_sharded_typed<uint32_t>(g, sc, &v, sx, sy, sz, out, out_dtype, n_global);
+    case IGN_U64: return ccl_sharded_typed<uint64_t>(g, sc, &v, sx, sy, sz, out, out_dtype, n_global);
   }
-  scratch_reset(ctx);
-  return rc;
+  set_error("sharded CCL: unsupported input dtype %d", in_dtype);
+  return IGN_ERR_UNSUPPORTED;
 }
 
 }  // extern "C"

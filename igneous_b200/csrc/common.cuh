@@ -4,6 +4,7 @@
 #include <stdint.h>
 #include <stdio.h>
 #include <string>
+#include <vector>
 
 #include "../../include/igneous_b200.h"
 
@@ -52,7 +53,6 @@ static inline int dtype_size(int dt) {
 
 }  // namespace ign
 
-// grow-only device scratch arena, bump allocated per API call
 constexpr int IGN_TIMER_SLOTS = 64;  // CUDA event pairs per context: timers and cross-stream marks
 
 struct ign_ctx {
@@ -60,9 +60,13 @@ struct ign_ctx {
   int sm_count;
   cudaStream_t stream;
   cudaStream_t copy_stream;
+  // grow-only device scratch arena, bump allocated through ign::Scratch
   char* scratch;
   size_t scratch_bytes;
   size_t scratch_used;
+  // grow-only device copies of the host-buffer entry points' arrays (ign::Staging)
+  char* stage;
+  size_t stage_bytes;
   char* pinned;  // staging for scalars / small results
   size_t pinned_bytes;
   cudaEvent_t timers[IGN_TIMER_SLOTS][2];
@@ -94,15 +98,75 @@ namespace ign {
 
 // Make `ctx->device` current (one ctx per process is the contract, but be safe).
 int activate(ign_ctx* ctx);
-// Reset the bump pointer; call at the start of every public API function.
-void scratch_reset(ign_ctx* ctx);
-// Bump-allocate `bytes` (256B aligned) from the arena.  The arena never moves
-// while allocations of the current call are alive: scratch_reserve() must be
-// called first with the total the call needs.
-int scratch_reserve(ign_ctx* ctx, size_t total_bytes);
-void* scratch_take(ign_ctx* ctx, size_t bytes);
 
 static inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
+
+// Grow a grow-only device buffer to at least `need` bytes (plus a quarter, so that slowly rising
+// sizes do not reallocate every call).  The contents are dropped; work queued on ctx->stream is
+// waited for first, since it may still use the old buffer.
+int grow_buffer(ign_ctx* ctx, char** buf, size_t* have, size_t need, const char* what);
+
+// One function's use of the scratch arena.  Construct it at the top of every function that takes
+// from the arena; its destructor gives the bytes back on every return path.  The scope owns the
+// arena iff nothing is held below it: the outermost call, with no CCL volume open.  Only the owner
+// grows the arena, since growing moves it; a nested scope lives in the room its caller reserved.
+class Scratch {
+ public:
+  explicit Scratch(ign_ctx* ctx) : Scratch(ctx, ctx->scratch_used) {}
+  // adopts the bytes a kept scope with this base still holds: they are released with this scope
+  Scratch(ign_ctx* ctx, size_t base) : ctx_(ctx), base_(base) {}
+  ~Scratch() {
+    if (!kept_) ctx_->scratch_used = base_;
+  }
+  Scratch(const Scratch&) = delete;
+  Scratch& operator=(const Scratch&) = delete;
+
+  bool owner() const { return base_ == 0; }
+  // owner: make the arena at least `bytes` (call before the first take); nested: nothing
+  int reserve(size_t bytes);
+  // `count` elements, 256 B aligned; nullptr when they do not fit, and ok() turns false
+  template <typename T = char>
+  T* take(size_t count) { return (T*)take_bytes(count * sizeof(T)); }
+  bool ok() const { return ok_; }
+  // back to the base: every take of this scope is released
+  void rewind();
+  // leave the bytes held past this scope; returns the base to release them to later
+  size_t keep() {
+    kept_ = true;
+    return base_;
+  }
+
+ private:
+  void* take_bytes(size_t bytes);
+  ign_ctx* ctx_;
+  size_t base_;
+  bool ok_ = true, kept_ = false;
+};
+
+// Device copies of a host-buffer entry point's arrays, in the context's grow-only staging buffer.
+// They sit outside the scratch arena, so the _dev function the entry point calls sizes its own
+// arena use.  add() every slot, stage(), call the _dev function, back() its results, sync().
+class Staging {
+ public:
+  explicit Staging(ign_ctx* ctx) : ctx_(ctx) {}
+  // a device slot of `bytes` (nullptr if 0), filled from `host` unless that is null
+  void add(void** dev, size_t bytes, const void* host = nullptr) { slots_.push_back({dev, bytes, host}); }
+  // grows the buffer, sets every slot pointer and queues the host -> device copies
+  int stage();
+  // queues a device -> host copy of a result
+  int back(void* host, const void* dev, size_t bytes);
+  // waits for the copies
+  int sync();
+
+ private:
+  struct Slot {
+    void** dev;
+    size_t bytes;
+    const void* host;
+  };
+  ign_ctx* ctx_;
+  std::vector<Slot> slots_;
+};
 
 // Small control transfers (counters, per-label offset tables) that sit between kernels
 // of one call.  cudaMemcpyAsync would put them on a copy engine, where they queue behind

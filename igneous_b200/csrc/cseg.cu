@@ -294,8 +294,7 @@ static int cseg_encode_channel(ign_ctx* ctx, const T* in, const CsegDims& d, uin
                                uint64_t* n_words) {
   constexpr int WORDS = sizeof(T) / 4;
   const uint32_t nb = d.gx * d.gy * d.gz;
-  const size_t keep = ctx->scratch_used;
-  const bool own = keep == 0;
+  Scratch sc(ctx);
   size_t sortb = 0, scanb = 0;
   cub::DeviceRadixSort::SortPairs(nullptr, sortb, (const unsigned long long*)nullptr, (unsigned long long*)nullptr,
                                   (const uint32_t*)nullptr, (uint32_t*)nullptr, (int)nb);
@@ -306,98 +305,68 @@ static int cseg_encode_channel(ign_ctx* ctx, const T* in, const CsegDims& d, uin
     if (mb > scanb) scanb = mb;
   }
   const size_t tmpb = (sortb > scanb ? sortb : scanb) + 256;
-  if (own) IGN_TRY(scratch_reserve(ctx, 2 * align_up((size_t)nb * 8, 256) + 8 * align_up(((size_t)nb + 2) * 4, 256) + tmpb + 4096));
-  auto fail = [&](int rc) {
-    ctx->scratch_used = keep;
-    return rc;
-  };
-  unsigned long long* hash = (unsigned long long*)scratch_take(ctx, (size_t)nb * 8);
-  unsigned long long* shash = (unsigned long long*)scratch_take(ctx, (size_t)nb * 8);
-  uint32_t* n = (uint32_t*)scratch_take(ctx, ((size_t)nb + 1) * 4);
-  uint32_t* blk = (uint32_t*)scratch_take(ctx, ((size_t)nb + 1) * 4);
-  uint32_t* sblk = (uint32_t*)scratch_take(ctx, ((size_t)nb + 1) * 4);
-  uint32_t* owner = (uint32_t*)scratch_take(ctx, ((size_t)nb + 1) * 4);
-  uint32_t* size = (uint32_t*)scratch_take(ctx, ((size_t)nb + 1) * 4);
-  uint32_t* scan = (uint32_t*)scratch_take(ctx, ((size_t)nb + 2) * 4);  // [nb]: total, [nb + 1]: largest table offset
-  uint32_t* enc_off = (uint32_t*)scratch_take(ctx, ((size_t)nb + 1) * 4);
-  uint32_t* tab_off = (uint32_t*)scratch_take(ctx, ((size_t)nb + 1) * 4);
-  void* tmp = scratch_take(ctx, tmpb);
-  if (!hash || !shash || !n || !blk || !sblk || !owner || !size || !scan || !enc_off || !tab_off || !tmp) {
-    set_error("scratch arena too small (cseg encode)");
-    return fail(IGN_ERR_NOMEM);
-  }
-#define CS_CUDA(call)                                                                  \
-  do {                                                                                 \
-    cudaError_t _e = (call);                                                           \
-    if (_e != cudaSuccess) {                                                           \
-      set_error("%s:%d: %s -> %s", __FILE__, __LINE__, #call, cudaGetErrorString(_e)); \
-      return fail(IGN_ERR_CUDA);                                                       \
-    }                                                                                  \
-  } while (0)
-#define CS_LAUNCH(kernel, g, b, ...)                  \
-  do {                                                \
-    kernel<<<(g), (b), 0, ctx->stream>>>(__VA_ARGS__); \
-    ctx->launches++;                                  \
-    CS_CUDA(cudaGetLastError());                      \
-  } while (0)
+  IGN_TRY(sc.reserve(2 * align_up((size_t)nb * 8, 256) + 8 * align_up(((size_t)nb + 2) * 4, 256) + tmpb + 4096));
+  unsigned long long* hash = sc.take<unsigned long long>(nb);
+  unsigned long long* shash = sc.take<unsigned long long>(nb);
+  uint32_t* n = sc.take<uint32_t>((size_t)nb + 1);
+  uint32_t* blk = sc.take<uint32_t>((size_t)nb + 1);
+  uint32_t* sblk = sc.take<uint32_t>((size_t)nb + 1);
+  uint32_t* owner = sc.take<uint32_t>((size_t)nb + 1);
+  uint32_t* size = sc.take<uint32_t>((size_t)nb + 1);
+  uint32_t* scan = sc.take<uint32_t>((size_t)nb + 2);  // [nb]: total, [nb + 1]: largest table offset
+  uint32_t* enc_off = sc.take<uint32_t>((size_t)nb + 1);
+  uint32_t* tab_off = sc.take<uint32_t>((size_t)nb + 1);
+  void* tmp = sc.take(tmpb);
+  IGN_REQUIRE(sc.ok(), IGN_ERR_NOMEM, "scratch arena too small (cseg encode)");
   const unsigned gw = blocks_for((uint64_t)nb * 32, 128);
   if (d.bvox <= 512)
-    CS_LAUNCH((k_cseg_scan<T, false, 16>), gw, 128, in, d, (uint64_t)nb, n, hash, (const uint32_t*)nullptr,
+    IGN_LAUNCH(ctx, (k_cseg_scan<T, false, 16>), gw, 128, 0, in, d, (uint64_t)nb, n, hash, (const uint32_t*)nullptr,
               (const uint32_t*)nullptr, (const uint32_t*)nullptr, (uint32_t*)nullptr);
   else
-    CS_LAUNCH((k_cseg_scan<T, false, 32>), gw, 128, in, d, (uint64_t)nb, n, hash, (const uint32_t*)nullptr,
+    IGN_LAUNCH(ctx, (k_cseg_scan<T, false, 32>), gw, 128, 0, in, d, (uint64_t)nb, n, hash, (const uint32_t*)nullptr,
               (const uint32_t*)nullptr, (const uint32_t*)nullptr, (uint32_t*)nullptr);
-  CS_LAUNCH(k_iota32, blocks_for(nb, 256), 256, blk, nb);
+  IGN_LAUNCH(ctx, k_iota32, blocks_for(nb, 256), 256, 0, blk, nb);
   {
     size_t tb = tmpb;
-    CS_CUDA(cub::DeviceRadixSort::SortPairs(tmp, tb, hash, shash, blk, sblk, (int)nb, 0, 64, ctx->stream));
+    IGN_CUDA(cub::DeviceRadixSort::SortPairs(tmp, tb, hash, shash, blk, sblk, (int)nb, 0, 64, ctx->stream));
     ctx->launches += 9;
   }
-  CS_LAUNCH(k_cseg_heads, blocks_for(nb, 256), 256, shash, nb, enc_off);  // enc_off / tab_off: free until the offsets pass
+  IGN_LAUNCH(ctx, k_cseg_heads, blocks_for(nb, 256), 256, 0, shash, nb, enc_off);  // enc_off / tab_off: free until the offsets pass
   {
     size_t tb = tmpb;
-    CS_CUDA(cub::DeviceScan::InclusiveScan(tmp, tb, enc_off, tab_off, cub::Max(), (int)nb, ctx->stream));
+    IGN_CUDA(cub::DeviceScan::InclusiveScan(tmp, tb, enc_off, tab_off, cub::Max(), (int)nb, ctx->stream));
     ctx->launches += 2;
   }
   if (d.bvox <= 512)
-    CS_LAUNCH((k_cseg_owner<T, 16>), gw, 128, in, d, tab_off, sblk, n, nb, owner);
+    IGN_LAUNCH(ctx, (k_cseg_owner<T, 16>), gw, 128, 0, in, d, tab_off, sblk, n, nb, owner);
   else
-    CS_LAUNCH((k_cseg_owner<T, 32>), gw, 128, in, d, tab_off, sblk, n, nb, owner);
-  CS_LAUNCH((k_cseg_sizes<WORDS>), blocks_for(nb, 256), 256, n, owner, nb, d.bvox, size);
-  CS_CUDA(cudaMemsetAsync(size + nb, 0, 4, ctx->stream));
+    IGN_LAUNCH(ctx, (k_cseg_owner<T, 32>), gw, 128, 0, in, d, tab_off, sblk, n, nb, owner);
+  IGN_LAUNCH(ctx, (k_cseg_sizes<WORDS>), blocks_for(nb, 256), 256, 0, n, owner, nb, d.bvox, size);
+  IGN_CUDA(cudaMemsetAsync(size + nb, 0, 4, ctx->stream));
   {
     size_t tb = tmpb;
-    CS_CUDA(cub::DeviceScan::ExclusiveSum(tmp, tb, size, scan, (int)nb + 1, ctx->stream));
+    IGN_CUDA(cub::DeviceScan::ExclusiveSum(tmp, tb, size, scan, (int)nb + 1, ctx->stream));
     ctx->launches += 2;
   }
-  CS_CUDA(cudaMemsetAsync(scan + nb + 1, 0, 4, ctx->stream));
-  CS_LAUNCH(k_cseg_offsets, blocks_for(nb, 256), 256, n, owner, scan, nb, d.bvox, enc_off, tab_off, scan + nb + 1);
+  IGN_CUDA(cudaMemsetAsync(scan + nb + 1, 0, 4, ctx->stream));
+  IGN_LAUNCH(ctx, k_cseg_offsets, blocks_for(nb, 256), 256, 0, n, owner, scan, nb, d.bvox, enc_off, tab_off, scan + nb + 1);
   uint32_t tail[2] = {0, 0};  // words after the headers, largest table offset
-  {
-    const int rc = small_d2h(ctx, tail, scan + nb, 8);
-    if (rc != IGN_OK) return fail(rc);
-    const int rc2 = small_sync(ctx);
-    if (rc2 != IGN_OK) return fail(rc2);
-  }
+  IGN_TRY(small_d2h(ctx, tail, scan + nb, 8));
+  IGN_TRY(small_sync(ctx));
   const uint64_t words = 2ull * nb + tail[0];
   *n_words = words;
-  if (tail[1] > 0xFFFFFFu) {
-    set_error("cseg: a lookup table of the encoded chunk starts at word %u, beyond the format's 24-bit table offsets",
+  IGN_REQUIRE(tail[1] <= 0xFFFFFFu, IGN_ERR_OVERFLOW,
+              "cseg: a lookup table of the encoded chunk starts at word %u, beyond the format's 24-bit table offsets",
               tail[1]);
-    return fail(IGN_ERR_OVERFLOW);
-  }
   if (out_dev != nullptr && words <= cap_words) {
     if (d.bvox <= 512)
-      CS_LAUNCH((k_cseg_scan<T, true, 16>), gw, 128, in, d, (uint64_t)nb, (uint32_t*)nullptr, (unsigned long long*)nullptr,
+      IGN_LAUNCH(ctx, (k_cseg_scan<T, true, 16>), gw, 128, 0, in, d, (uint64_t)nb, (uint32_t*)nullptr, (unsigned long long*)nullptr,
                 enc_off, tab_off, owner, out_dev);
     else
-      CS_LAUNCH((k_cseg_scan<T, true, 32>), gw, 128, in, d, (uint64_t)nb, (uint32_t*)nullptr, (unsigned long long*)nullptr,
+      IGN_LAUNCH(ctx, (k_cseg_scan<T, true, 32>), gw, 128, 0, in, d, (uint64_t)nb, (uint32_t*)nullptr, (unsigned long long*)nullptr,
                 enc_off, tab_off, owner, out_dev);
   }
-  ctx->scratch_used = keep;
   return IGN_OK;
-#undef CS_CUDA
-#undef CS_LAUNCH
 }
 
 }  // namespace ign
@@ -443,18 +412,14 @@ int ign_cseg_decode_dev(ign_ctx* ctx, const uint32_t* in, uint64_t n_words, int 
   std::vector<uint32_t> chan_off(sc, 0);
   IGN_CUDA(cudaMemcpyAsync(chan_off.data(), in, sc * 4, cudaMemcpyDeviceToHost, ctx->stream));
   IGN_CUDA(cudaStreamSynchronize(ctx->stream));
-  const size_t keep = ctx->scratch_used;
-  if (keep == 0) IGN_TRY(scratch_reserve(ctx, 4096));
-  uint32_t* err = (uint32_t*)scratch_take(ctx, 256);
-  IGN_REQUIRE(err != nullptr, IGN_ERR_NOMEM, "scratch arena too small (cseg decode)");
+  Scratch arena(ctx);  // `sc` is the channel count here
+  IGN_TRY(arena.reserve(4096));
+  uint32_t* err = arena.take<uint32_t>(64);
+  IGN_REQUIRE(arena.ok(), IGN_ERR_NOMEM, "scratch arena too small (cseg decode)");
   IGN_CUDA(cudaMemsetAsync(err, 0, 4, ctx->stream));
   for (uint64_t c = 0; c < sc; c++) {
     const uint64_t base = chan_off[c];
-    if (base > n_words) {
-      ctx->scratch_used = keep;
-      set_error("cseg: channel offset outside the stream");
-      return IGN_ERR_INVALID;
-    }
+    IGN_REQUIRE(base <= n_words, IGN_ERR_INVALID, "cseg: channel offset outside the stream");
     if (dtype == IGN_U32)
       IGN_LAUNCH(ctx, (k_cseg_decode<uint32_t>), blocks_for(n, 256), 256, 0, in + base, n_words - base, d, (uint32_t*)out + c * n, err);
     else
@@ -463,7 +428,6 @@ int ign_cseg_decode_dev(ign_ctx* ctx, const uint32_t* in, uint64_t n_words, int 
   uint32_t herr = 0;
   IGN_CUDA(cudaMemcpyAsync(&herr, err, 4, cudaMemcpyDeviceToHost, ctx->stream));
   IGN_CUDA(cudaStreamSynchronize(ctx->stream));
-  ctx->scratch_used = keep;
   IGN_REQUIRE(herr == 0, IGN_ERR_INVALID, "cseg: malformed stream");
   return IGN_OK;
 }
@@ -476,24 +440,14 @@ int ign_cseg_encode(ign_ctx* ctx, const void* labels, int dtype, uint64_t sx, ui
   IGN_REQUIRE(labels && n_words, IGN_ERR_INVALID, "null argument");
   const int es = dtype_size(dtype);
   IGN_REQUIRE(dtype == IGN_U32 || dtype == IGN_U64, IGN_ERR_UNSUPPORTED, "compressed_segmentation holds uint32 / uint64 labels");
-  const uint64_t n = sx * sy * sz * sc;
-  scratch_reset(ctx);
-  IGN_TRY(scratch_reserve(ctx, align_up(n * es, 256) + align_up((out ? cap_words : 0) * 4, 256) + (64ull << 20)));
-  void* d_in = scratch_take(ctx, n * es);
-  uint32_t* d_out = out ? (uint32_t*)scratch_take(ctx, cap_words * 4) : nullptr;
-  IGN_REQUIRE(d_in && (!out || d_out), IGN_ERR_NOMEM, "scratch arena too small (cseg)");
-  IGN_CUDA(cudaMemcpyAsync(d_in, labels, n * es, cudaMemcpyHostToDevice, ctx->stream));
-  int rc = ign_cseg_encode_dev(ctx, d_in, dtype, sx, sy, sz, sc, bx, by, bz, d_out, cap_words, n_words);
-  if (rc == IGN_OK && out && *n_words <= cap_words) {
-    cudaError_t e = cudaMemcpyAsync(out, d_out, *n_words * 4, cudaMemcpyDeviceToHost, ctx->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-    if (e != cudaSuccess) {
-      set_error("cseg D2H: %s", cudaGetErrorString(e));
-      rc = IGN_ERR_CUDA;
-    }
-  }
-  scratch_reset(ctx);
-  return rc;
+  Staging st(ctx);
+  void *d_in, *d_out;
+  st.add(&d_in, sx * sy * sz * sc * es, labels);
+  st.add(&d_out, out ? cap_words * 4 : 0);
+  IGN_TRY(st.stage());
+  IGN_TRY(ign_cseg_encode_dev(ctx, d_in, dtype, sx, sy, sz, sc, bx, by, bz, (uint32_t*)d_out, cap_words, n_words));
+  if (out && *n_words <= cap_words) IGN_TRY(st.back(out, d_out, *n_words * 4));
+  return st.sync();
 }
 
 int ign_cseg_decode(ign_ctx* ctx, const uint32_t* in, uint64_t n_words, int dtype, uint64_t sx, uint64_t sy, uint64_t sz,
@@ -503,23 +457,14 @@ int ign_cseg_decode(ign_ctx* ctx, const uint32_t* in, uint64_t n_words, int dtyp
   const int es = dtype_size(dtype);
   IGN_REQUIRE(dtype == IGN_U32 || dtype == IGN_U64, IGN_ERR_UNSUPPORTED, "compressed_segmentation holds uint32 / uint64 labels");
   const uint64_t n = sx * sy * sz * sc;
-  scratch_reset(ctx);
-  IGN_TRY(scratch_reserve(ctx, align_up(n * es, 256) + align_up(n_words * 4, 256) + (1 << 20)));
-  uint32_t* d_in = (uint32_t*)scratch_take(ctx, n_words * 4);
-  void* d_out = scratch_take(ctx, n * es);
-  IGN_REQUIRE(d_in && d_out, IGN_ERR_NOMEM, "scratch arena too small (cseg)");
-  IGN_CUDA(cudaMemcpyAsync(d_in, in, n_words * 4, cudaMemcpyHostToDevice, ctx->stream));
-  int rc = ign_cseg_decode_dev(ctx, d_in, n_words, dtype, sx, sy, sz, sc, bx, by, bz, d_out);
-  if (rc == IGN_OK) {
-    cudaError_t e = cudaMemcpyAsync(out, d_out, n * es, cudaMemcpyDeviceToHost, ctx->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-    if (e != cudaSuccess) {
-      set_error("cseg D2H: %s", cudaGetErrorString(e));
-      rc = IGN_ERR_CUDA;
-    }
-  }
-  scratch_reset(ctx);
-  return rc;
+  Staging st(ctx);
+  void *d_in, *d_out;
+  st.add(&d_in, n_words * 4, in);
+  st.add(&d_out, n * es);
+  IGN_TRY(st.stage());
+  IGN_TRY(ign_cseg_decode_dev(ctx, (const uint32_t*)d_in, n_words, dtype, sx, sy, sz, sc, bx, by, bz, d_out));
+  IGN_TRY(st.back(out, d_out, n * es));
+  return st.sync();
 }
 
 }  // extern "C"

@@ -23,30 +23,70 @@ int activate(ign_ctx* ctx) {
   return IGN_OK;
 }
 
-void scratch_reset(ign_ctx* ctx) { ctx->scratch_used = 0; }
-
-int scratch_reserve(ign_ctx* ctx, size_t total) {
-  total = align_up(total + 4096, 1 << 20);
-  if (total <= ctx->scratch_bytes) return IGN_OK;
+// replaces *buf by a fresh allocation of exactly `bytes`
+static int realloc_buffer(ign_ctx* ctx, char** buf, size_t* have, size_t bytes, const char* what) {
   IGN_CUDA(cudaStreamSynchronize(ctx->stream));
-  if (ctx->scratch) IGN_CUDA(cudaFree(ctx->scratch));
-  ctx->scratch = nullptr;
-  ctx->scratch_bytes = 0;
-  cudaError_t e = cudaMalloc((void**)&ctx->scratch, total);
+  if (*buf) IGN_CUDA(cudaFree(*buf));
+  *buf = nullptr;
+  *have = 0;
+  cudaError_t e = cudaMalloc((void**)buf, bytes);
   if (e != cudaSuccess) {
     cudaGetLastError();
-    set_error("scratch arena: cudaMalloc(%zu) failed: %s", total, cudaGetErrorString(e));
+    set_error("%s: cudaMalloc(%zu) failed: %s", what, bytes, cudaGetErrorString(e));
     return IGN_ERR_NOMEM;
   }
-  ctx->scratch_bytes = total;
+  *have = bytes;
   return IGN_OK;
 }
 
-void* scratch_take(ign_ctx* ctx, size_t bytes) {
-  size_t off = align_up(ctx->scratch_used, 256);
-  if (off + bytes > ctx->scratch_bytes) return nullptr;
-  ctx->scratch_used = off + bytes;
-  return ctx->scratch + off;
+int grow_buffer(ign_ctx* ctx, char** buf, size_t* have, size_t need, const char* what) {
+  if (*have >= need) return IGN_OK;
+  return realloc_buffer(ctx, buf, have, need + need / 4, what);
+}
+
+int Scratch::reserve(size_t bytes) {
+  if (!owner()) return IGN_OK;
+  bytes = align_up(bytes + 4096, 1 << 20);
+  if (bytes <= ctx_->scratch_bytes) return IGN_OK;
+  return realloc_buffer(ctx_, &ctx_->scratch, &ctx_->scratch_bytes, bytes, "scratch arena");
+}
+
+void* Scratch::take_bytes(size_t bytes) {
+  const size_t off = align_up(ctx_->scratch_used, 256);
+  if (off + bytes > ctx_->scratch_bytes) {
+    ok_ = false;
+    return nullptr;
+  }
+  ctx_->scratch_used = off + bytes;
+  return ctx_->scratch + off;
+}
+
+void Scratch::rewind() {
+  ctx_->scratch_used = base_;
+  ok_ = true;
+}
+
+int Staging::stage() {
+  size_t total = 0;
+  for (const Slot& s : slots_) total += align_up(s.bytes, 256);
+  IGN_TRY(grow_buffer(ctx_, &ctx_->stage, &ctx_->stage_bytes, total, "staging buffer"));
+  size_t off = 0;
+  for (const Slot& s : slots_) {
+    *s.dev = s.bytes ? ctx_->stage + off : nullptr;
+    if (s.host && s.bytes) IGN_CUDA(cudaMemcpyAsync(*s.dev, s.host, s.bytes, cudaMemcpyHostToDevice, ctx_->stream));
+    off += align_up(s.bytes, 256);
+  }
+  return IGN_OK;
+}
+
+int Staging::back(void* host, const void* dev, size_t bytes) {
+  if (bytes) IGN_CUDA(cudaMemcpyAsync(host, dev, bytes, cudaMemcpyDeviceToHost, ctx_->stream));
+  return IGN_OK;
+}
+
+int Staging::sync() {
+  IGN_CUDA(cudaStreamSynchronize(ctx_->stream));
+  return IGN_OK;
 }
 
 template <typename T>
@@ -213,6 +253,8 @@ int ign_init(int device, ign_ctx** out) {
   ctx->sm_count = prop.multiProcessorCount;
   ctx->scratch = nullptr;
   ctx->scratch_bytes = ctx->scratch_used = 0;
+  ctx->stage = nullptr;
+  ctx->stage_bytes = 0;
   ctx->launches = 0;
   ctx->prof_on = 0;
   ctx->prof = nullptr;
@@ -248,6 +290,7 @@ int ign_destroy(ign_ctx* ctx) {
   cudaSetDevice(ctx->device);
   cudaStreamSynchronize(ctx->stream);
   if (ctx->scratch) cudaFree(ctx->scratch);
+  if (ctx->stage) cudaFree(ctx->stage);
   if (ctx->pinned) cudaFreeHost(ctx->pinned);
   if (ctx->win) cudaFreeHost(ctx->win);
   if (ctx->mesh_pool) cudaFree(ctx->mesh_pool);

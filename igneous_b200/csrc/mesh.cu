@@ -23,6 +23,7 @@
 #include <cub/device/device_scan.cuh>
 
 #include <atomic>
+#include <memory>
 #include <vector>
 
 #include "common.cuh"
@@ -280,6 +281,11 @@ int ign_mesh_free(ign_mesher* m) {
   return IGN_OK;
 }
 
+// frees a mesher that ign_mesh_begin_dev could not finish
+struct MesherFree {
+  void operator()(ign_mesher* m) const { ign_mesh_free(m); }
+};
+
 int ign_mesh_begin_dev(ign_ctx* ctx, const void* labels, int dtype, uint64_t sx, uint64_t sy,
                        uint64_t sz, ign_mesher** out) {
   IGN_TRY(activate(ctx));
@@ -291,10 +297,9 @@ int ign_mesh_begin_dev(ign_ctx* ctx, const void* labels, int dtype, uint64_t sx,
               (unsigned long long)sx, (unsigned long long)sy, (unsigned long long)sz);
   IGN_TRY(load_tables(ctx));
   const uint64_t n = sx * sy * sz;
-  const bool own = (ctx->scratch_used == 0);
-  const size_t keep = ctx->scratch_used;
+  Scratch sc(ctx);
 
-  ign_mesher* m = new ign_mesher();
+  std::unique_ptr<ign_mesher, MesherFree> m(new ign_mesher());
   m->ctx = ctx;
   m->K = m->T = m->U = 0;
   m->d_uniq_vkeys = nullptr;
@@ -305,91 +310,50 @@ int ign_mesh_begin_dev(ign_ctx* ctx, const void* labels, int dtype, uint64_t sx,
   m->simp_factor = 0;
   m->simp_max_error = 0;
   m->simp_rounds = 0;
-  int rc = IGN_OK;
-  auto fail = [&](int code) {
-    ctx->scratch_used = keep;
-    ign_mesh_free(m);
-    return code;
-  };
 
   // ---- dense labels
   uint64_t cap2 = 1024;
   while (cap2 < 2 * n + 16 && cap2 < (1ull << 31)) cap2 <<= 1;
   const size_t renumber_need = cap2 * 40 + (1 << 20);
-  if (own) {
-    rc = scratch_reserve(ctx, align_up(n * 4, 256) + align_up(n * 8, 256) + renumber_need + (64 << 20));
-    if (rc != IGN_OK) return fail(rc);
-  }
-  uint32_t* d_lab = (uint32_t*)scratch_take(ctx, n * 4);
-  uint64_t* d_uniq = (uint64_t*)scratch_take(ctx, n * 8);
-  if (!d_lab || !d_uniq) {
-    set_error("scratch arena too small (mesher labels)");
-    return fail(IGN_ERR_NOMEM);
-  }
+  IGN_TRY(sc.reserve(align_up(n * 4, 256) + align_up(n * 8, 256) + renumber_need + (64 << 20)));
+  uint32_t* d_lab = sc.take<uint32_t>(n);
+  uint64_t* d_uniq = sc.take<uint64_t>(n);
+  IGN_REQUIRE(sc.ok(), IGN_ERR_NOMEM, "scratch arena too small (mesher labels)");
   uint64_t K = 0;
-  rc = ign_renumber_dev(ctx, labels, dtype, n, d_lab, d_uniq, n, &K);
-  if (rc != IGN_OK) return fail(rc);
+  IGN_TRY(ign_renumber_dev(ctx, labels, dtype, n, d_lab, d_uniq, n, &K));
   m->K = K;
   m->ids.resize(K);
   if (K) {
-    rc = small_d2h(ctx, m->ids.data(), d_uniq, K * 8);
-    if (rc == IGN_OK) rc = small_sync(ctx);
-    if (rc != IGN_OK) return fail(rc);
+    IGN_TRY(small_d2h(ctx, m->ids.data(), d_uniq, K * 8));
+    IGN_TRY(small_sync(ctx));
   }
   m->tri_off.assign(K + 2, 0);
   m->vert_off.assign(K + 2, 0);
   if (K == 0 || sx < 2 || sy < 2 || sz < 2) {
-    ctx->scratch_used = keep;
-    *out = m;
+    *out = m.release();
     return IGN_OK;
   }
-  if (K >= (1ull << 31)) {
-    set_error("mesher: too many labels");
-    return fail(IGN_ERR_OVERFLOW);
-  }
+  IGN_REQUIRE(K < (1ull << 31), IGN_ERR_OVERFLOW, "mesher: too many labels");
   // the arena below d_uniq is reusable now: only d_lab must survive
-  ctx->scratch_used = keep;
-  d_lab = (uint32_t*)scratch_take(ctx, n * 4);
+  sc.rewind();
+  d_lab = sc.take<uint32_t>(n);
 
   // ---- count
-  unsigned long long* d_total = (unsigned long long*)scratch_take(ctx, 256);
+  unsigned long long* d_total = sc.take<unsigned long long>(32);
   const uint64_t ncubes = (sx - 1) * (sy - 1) * (sz - 1);
   const unsigned grid = blocks_for(ncubes, 256);
   unsigned long long T = 0;
-#define MESH_CUDA(call)                                                            \
-  do {                                                                             \
-    cudaError_t _e = (call);                                                       \
-    if (_e != cudaSuccess) {                                                       \
-      set_error("%s:%d: %s -> %s", __FILE__, __LINE__, #call, cudaGetErrorString(_e)); \
-      return fail(IGN_ERR_CUDA);                                                   \
-    }                                                                              \
-  } while (0)
-#define MESH_TRY(call)                    \
-  do {                                    \
-    const int _s = (call);                \
-    if (_s != IGN_OK) return fail(_s);    \
-  } while (0)
-#define MESH_LAUNCH(kernel, g, b, ...)                    \
-  do {                                                    \
-    kernel<<<(g), (b), 0, ctx->stream>>>(__VA_ARGS__);    \
-    ctx->launches++;                                      \
-    MESH_CUDA(cudaGetLastError());                        \
-  } while (0)
-  MESH_CUDA(cudaMemsetAsync(d_total, 0, 8, ctx->stream));
-  MESH_LAUNCH((k_mc<false>), grid, 256, d_lab, (uint32_t)sx, (uint32_t)sy, (uint32_t)sz, d_total,
-              (uint64_t*)nullptr, (uint8_t*)nullptr, 0ull);
-  MESH_TRY(small_d2h(ctx, &T, d_total, 8));
-  MESH_TRY(small_sync(ctx));
+  IGN_CUDA(cudaMemsetAsync(d_total, 0, 8, ctx->stream));
+  IGN_LAUNCH(ctx, (k_mc<false>), grid, 256, 0, d_lab, (uint32_t)sx, (uint32_t)sy, (uint32_t)sz, d_total,
+             (uint64_t*)nullptr, (uint8_t*)nullptr, 0ull);
+  IGN_TRY(small_d2h(ctx, &T, d_total, 8));
+  IGN_TRY(small_sync(ctx));
   m->T = T;
   if (T == 0) {
-    ctx->scratch_used = keep;
-    *out = m;
+    *out = m.release();
     return IGN_OK;
   }
-  if (3 * T >= 0xFFFFFFFFull) {
-    set_error("mesher: %llu triangles exceed 32-bit corner indices", T);
-    return fail(IGN_ERR_OVERFLOW);
-  }
+  IGN_REQUIRE(3 * T < 0xFFFFFFFFull, IGN_ERR_OVERFLOW, "mesher: %llu triangles exceed 32-bit corner indices", T);
 
   // ---- arena plan for emit + sort + weld
   size_t sort1 = 0, sort2 = 0, scanb = 0;
@@ -403,110 +367,95 @@ int ign_mesh_begin_dev(ign_ctx* ctx, const void* labels, int dtype, uint64_t sx,
   const size_t need = align_up(n * 4, 256) + 2 * align_up(T * 8, 256) + 2 * align_up(T, 256) +
                       2 * align_up(3 * T * 8, 256) + 4 * align_up(3 * T * 4, 256) +
                       2 * align_up((K + 2) * 4, 256) + tmp_bytes + (1 << 20);
-  if (own && need > ctx->scratch_bytes) {
+  if (sc.owner() && need > ctx->scratch_bytes) {
     // growing the arena invalidates d_lab: re-run the (cheap) renumber into the new arena
-    ctx->scratch_used = keep;
-    rc = scratch_reserve(ctx, need + renumber_need + align_up(n * 8, 256));
-    if (rc != IGN_OK) return fail(rc);
-    d_lab = (uint32_t*)scratch_take(ctx, n * 4);
-    uint64_t* d_uniq2 = (uint64_t*)scratch_take(ctx, n * 8);
+    sc.rewind();
+    IGN_TRY(sc.reserve(need + renumber_need + align_up(n * 8, 256)));
+    d_lab = sc.take<uint32_t>(n);
+    uint64_t* d_uniq2 = sc.take<uint64_t>(n);
     uint64_t K2 = 0;
-    rc = ign_renumber_dev(ctx, labels, dtype, n, d_lab, d_uniq2, n, &K2);
-    if (rc != IGN_OK) return fail(rc);
-    ctx->scratch_used = keep;
-    d_lab = (uint32_t*)scratch_take(ctx, n * 4);
-    d_total = (unsigned long long*)scratch_take(ctx, 256);
+    IGN_TRY(ign_renumber_dev(ctx, labels, dtype, n, d_lab, d_uniq2, n, &K2));
+    sc.rewind();
+    d_lab = sc.take<uint32_t>(n);
+    d_total = sc.take<unsigned long long>(32);
   }
-  uint64_t* keys = (uint64_t*)scratch_take(ctx, T * 8);
-  uint64_t* keys_s = (uint64_t*)scratch_take(ctx, T * 8);
-  uint8_t* cases = (uint8_t*)scratch_take(ctx, T);
-  uint8_t* cases_s = (uint8_t*)scratch_take(ctx, T);
-  uint64_t* vkeys = (uint64_t*)scratch_take(ctx, 3 * T * 8);
-  uint64_t* vkeys_s = (uint64_t*)scratch_take(ctx, 3 * T * 8);
-  uint32_t* corner = (uint32_t*)scratch_take(ctx, 3 * T * 4);
-  uint32_t* corner_s = (uint32_t*)scratch_take(ctx, 3 * T * 4);
-  uint32_t* heads = (uint32_t*)scratch_take(ctx, 3 * T * 4);
-  uint32_t* rank = (uint32_t*)scratch_take(ctx, 3 * T * 4);
-  uint32_t* d_tri_off = (uint32_t*)scratch_take(ctx, (K + 2) * 4);
-  uint32_t* d_vert_off = (uint32_t*)scratch_take(ctx, (K + 2) * 4);
-  void* tmp = scratch_take(ctx, tmp_bytes);
-  if (!keys || !keys_s || !cases || !cases_s || !vkeys || !vkeys_s || !corner || !corner_s || !heads ||
-      !rank || !d_tri_off || !d_vert_off || !tmp) {
-    set_error("scratch arena too small (mesher: %llu triangles)", T);
-    return fail(IGN_ERR_NOMEM);
-  }
+  uint64_t* keys = sc.take<uint64_t>(T);
+  uint64_t* keys_s = sc.take<uint64_t>(T);
+  uint8_t* cases = sc.take<uint8_t>(T);
+  uint8_t* cases_s = sc.take<uint8_t>(T);
+  uint64_t* vkeys = sc.take<uint64_t>(3 * T);
+  uint64_t* vkeys_s = sc.take<uint64_t>(3 * T);
+  uint32_t* corner = sc.take<uint32_t>(3 * T);
+  uint32_t* corner_s = sc.take<uint32_t>(3 * T);
+  uint32_t* heads = sc.take<uint32_t>(3 * T);
+  uint32_t* rank = sc.take<uint32_t>(3 * T);
+  uint32_t* d_tri_off = sc.take<uint32_t>(K + 2);
+  uint32_t* d_vert_off = sc.take<uint32_t>(K + 2);
+  void* tmp = sc.take(tmp_bytes);
+  IGN_REQUIRE(sc.ok(), IGN_ERR_NOMEM, "scratch arena too small (mesher: %llu triangles)", T);
 
   // ---- emit + sort
-  MESH_CUDA(cudaMemsetAsync(d_total, 0, 8, ctx->stream));
-  MESH_LAUNCH((k_mc<true>), grid, 256, d_lab, (uint32_t)sx, (uint32_t)sy, (uint32_t)sz, d_total, keys,
-              cases, (uint64_t)T);
+  IGN_CUDA(cudaMemsetAsync(d_total, 0, 8, ctx->stream));
+  IGN_LAUNCH(ctx, (k_mc<true>), grid, 256, 0, d_lab, (uint32_t)sx, (uint32_t)sy, (uint32_t)sz, d_total, keys,
+             cases, (uint64_t)T);
   const int label_bits = bits_for(K);
   size_t tb = tmp_bytes;
-  MESH_CUDA(cub::DeviceRadixSort::SortPairs(tmp, tb, keys, keys_s, cases, cases_s, (int)T, 0,
-                                            TRI_LABEL_SHIFT + label_bits, ctx->stream));
+  IGN_CUDA(cub::DeviceRadixSort::SortPairs(tmp, tb, keys, keys_s, cases, cases_s, (int)T, 0,
+                                           TRI_LABEL_SHIFT + label_bits, ctx->stream));
   ctx->launches += 4;
 
   // ---- weld
-  MESH_LAUNCH(k_tri_vertices, blocks_for(T, 256), 256, keys_s, cases_s, (uint64_t)T, (uint32_t)(sx - 1),
-              (uint32_t)(sy - 1), vkeys, corner);
+  IGN_LAUNCH(ctx, k_tri_vertices, blocks_for(T, 256), 256, 0, keys_s, cases_s, (uint64_t)T, (uint32_t)(sx - 1),
+             (uint32_t)(sy - 1), vkeys, corner);
   tb = tmp_bytes;
-  MESH_CUDA(cub::DeviceRadixSort::SortPairs(tmp, tb, vkeys, vkeys_s, corner, corner_s, (int)(3 * T), 0,
-                                            V_LABEL_SHIFT + label_bits, ctx->stream));
+  IGN_CUDA(cub::DeviceRadixSort::SortPairs(tmp, tb, vkeys, vkeys_s, corner, corner_s, (int)(3 * T), 0,
+                                           V_LABEL_SHIFT + label_bits, ctx->stream));
   ctx->launches += 4;
-  MESH_LAUNCH(k_vertex_heads, blocks_for(3 * T, 256), 256, vkeys_s, (uint64_t)(3 * T), heads);
+  IGN_LAUNCH(ctx, k_vertex_heads, blocks_for(3 * T, 256), 256, 0, vkeys_s, (uint64_t)(3 * T), heads);
   tb = tmp_bytes;
-  MESH_CUDA(cub::DeviceScan::ExclusiveSum(tmp, tb, heads, rank, (int)(3 * T), ctx->stream));
+  IGN_CUDA(cub::DeviceScan::ExclusiveSum(tmp, tb, heads, rank, (int)(3 * T), ctx->stream));
   ctx->launches += 2;
   uint32_t last[2];
-  MESH_TRY(small_d2h(ctx, &last[0], rank + (3 * T - 1), 4));
-  MESH_TRY(small_d2h(ctx, &last[1], heads + (3 * T - 1), 4));
-  MESH_TRY(small_sync(ctx));
+  IGN_TRY(small_d2h(ctx, &last[0], rank + (3 * T - 1), 4));
+  IGN_TRY(small_d2h(ctx, &last[1], heads + (3 * T - 1), 4));
+  IGN_TRY(small_sync(ctx));
   const uint64_t U = (uint64_t)last[0] + last[1];
   m->U = U;
   {
     const size_t fbytes = align_up(3 * T * 4, 256), vbytes = align_up(U * 12, 256);  // 12: float3 after simplify
     if (!ctx->mesh_pool_busy) {
-      if (ctx->mesh_pool_bytes < fbytes + vbytes) {
-        MESH_CUDA(cudaStreamSynchronize(ctx->stream));
-        if (ctx->mesh_pool) cudaFree(ctx->mesh_pool);
-        ctx->mesh_pool = nullptr;
-        ctx->mesh_pool_bytes = 0;
-        const size_t want = (fbytes + vbytes) * 5 / 4;
-        MESH_CUDA(cudaMalloc((void**)&ctx->mesh_pool, want));
-        ctx->mesh_pool_bytes = want;
-      }
+      IGN_TRY(grow_buffer(ctx, &ctx->mesh_pool, &ctx->mesh_pool_bytes, fbytes + vbytes, "mesh pool"));
       m->d_faces = (uint32_t*)ctx->mesh_pool;
       m->d_uniq_vkeys = (uint64_t*)(ctx->mesh_pool + fbytes);
       m->pooled = true;
       ctx->mesh_pool_busy = 1;
     } else {
-      MESH_CUDA(cudaMalloc((void**)&m->d_faces, 3 * T * 4));
-      MESH_CUDA(cudaMalloc((void**)&m->d_uniq_vkeys, U * 12));  // 12: float3 positions after simplification
+      IGN_CUDA(cudaMalloc((void**)&m->d_faces, 3 * T * 4));
+      IGN_CUDA(cudaMalloc((void**)&m->d_uniq_vkeys, U * 12));  // 12: float3 positions after simplification
     }
   }
-  MESH_LAUNCH(k_vertex_assign, blocks_for(3 * T, 256), 256, vkeys_s, corner_s, heads, rank,
-              (uint64_t)(3 * T), m->d_uniq_vkeys, m->d_faces);
+  IGN_LAUNCH(ctx, k_vertex_assign, blocks_for(3 * T, 256), 256, 0, vkeys_s, corner_s, heads, rank,
+             (uint64_t)(3 * T), m->d_uniq_vkeys, m->d_faces);
 
   // ---- per-label offsets (labels are 1..K; slot K+1 is the end sentinel)
-  MESH_LAUNCH(k_fill_u32, blocks_for(K + 2, 256), 256, d_tri_off, (uint32_t)T, (uint32_t)(K + 2));
-  MESH_LAUNCH(k_fill_u32, blocks_for(K + 2, 256), 256, d_vert_off, (uint32_t)U, (uint32_t)(K + 2));
-  MESH_LAUNCH(k_label_starts, blocks_for(T, 256), 256, keys_s, (uint64_t)T, TRI_LABEL_SHIFT, d_tri_off);
-  MESH_LAUNCH(k_label_starts, blocks_for(U, 256), 256, m->d_uniq_vkeys, U, V_LABEL_SHIFT, d_vert_off);
-  MESH_TRY(small_d2h(ctx, m->tri_off.data(), d_tri_off, (K + 2) * 4));
-  MESH_TRY(small_d2h(ctx, m->vert_off.data(), d_vert_off, (K + 2) * 4));
-  MESH_TRY(small_sync(ctx));
+  IGN_LAUNCH(ctx, k_fill_u32, blocks_for(K + 2, 256), 256, 0, d_tri_off, (uint32_t)T, (uint32_t)(K + 2));
+  IGN_LAUNCH(ctx, k_fill_u32, blocks_for(K + 2, 256), 256, 0, d_vert_off, (uint32_t)U, (uint32_t)(K + 2));
+  IGN_LAUNCH(ctx, k_label_starts, blocks_for(T, 256), 256, 0, keys_s, (uint64_t)T, TRI_LABEL_SHIFT, d_tri_off);
+  IGN_LAUNCH(ctx, k_label_starts, blocks_for(U, 256), 256, 0, m->d_uniq_vkeys, U, V_LABEL_SHIFT, d_vert_off);
+  IGN_TRY(small_d2h(ctx, m->tri_off.data(), d_tri_off, (K + 2) * 4));
+  IGN_TRY(small_d2h(ctx, m->vert_off.data(), d_vert_off, (K + 2) * 4));
+  IGN_TRY(small_sync(ctx));
   // absent labels hold the end marker: a suffix minimum turns starts into offsets
   for (int64_t l = (int64_t)K; l >= 0; l--) {
     if (m->tri_off[l] > m->tri_off[l + 1]) m->tri_off[l] = m->tri_off[l + 1];
     if (m->vert_off[l] > m->vert_off[l + 1]) m->vert_off[l] = m->vert_off[l + 1];
   }
-  MESH_TRY(small_h2d(ctx, d_vert_off, m->vert_off.data(), (K + 2) * 4));
-  MESH_LAUNCH(k_faces_local, blocks_for(3 * T, 256), 256, keys_s, d_vert_off, (uint64_t)T, m->d_faces);
-  MESH_CUDA(cudaStreamSynchronize(ctx->stream));
+  IGN_TRY(small_h2d(ctx, d_vert_off, m->vert_off.data(), (K + 2) * 4));
+  IGN_LAUNCH(ctx, k_faces_local, blocks_for(3 * T, 256), 256, 0, keys_s, d_vert_off, (uint64_t)T, m->d_faces);
+  IGN_CUDA(cudaStreamSynchronize(ctx->stream));
   for (uint64_t l = 1; l <= K; l++)
     if (m->tri_off[l + 1] > m->tri_off[l]) m->present.push_back(m->ids[l - 1]);
-  ctx->scratch_used = keep;
-  *out = m;
+  *out = m.release();
   return IGN_OK;
 }
 
@@ -516,22 +465,12 @@ int ign_mesh_begin(ign_ctx* ctx, const void* labels, int dtype, uint64_t sx, uin
   IGN_REQUIRE(labels && out, IGN_ERR_INVALID, "null argument");
   const int es = dtype_size(dtype);
   IGN_REQUIRE(es > 0 && dtype != IGN_F32, IGN_ERR_UNSUPPORTED, "unsupported dtype %d", dtype);
-  const uint64_t n = sx * sy * sz;
-  void* d = nullptr;
-  IGN_TRY(ign_dev_alloc(ctx, n * es, &d));
-  cudaError_t e = cudaMemcpyAsync(d, labels, n * es, cudaMemcpyHostToDevice, ctx->stream);
-  int rc = IGN_OK;
-  if (e != cudaSuccess) {
-    set_error("mesher H2D: %s", cudaGetErrorString(e));
-    rc = IGN_ERR_CUDA;
-  } else {
-    scratch_reset(ctx);
-    rc = ign_mesh_begin_dev(ctx, d, dtype, sx, sy, sz, out);
-    scratch_reset(ctx);
-  }
-  cudaStreamSynchronize(ctx->stream);
-  cudaFree(d);
-  return rc;
+  Staging st(ctx);
+  void* d;
+  st.add(&d, sx * sy * sz * es, labels);
+  IGN_TRY(st.stage());
+  IGN_TRY(ign_mesh_begin_dev(ctx, d, dtype, sx, sy, sz, out));
+  return st.sync();
 }
 
 int ign_mesh_num_ids(ign_mesher* m, uint64_t* n) {
@@ -577,10 +516,7 @@ int ign_mesh_get(ign_mesher* m, uint64_t id, const float resolution[3], int redu
   IGN_REQUIRE(m && resolution && nv && nf, IGN_ERR_INVALID, "null argument");
   ign_ctx* ctx = m->ctx;
   IGN_TRY(activate(ctx));
-  if (reduction_factor > 0 && !m->simplified) {
-    scratch_reset(ctx);
-    IGN_TRY(ign_mesh_simplify(m, resolution, reduction_factor, max_error));
-  }
+  if (reduction_factor > 0 && !m->simplified) IGN_TRY(ign_mesh_simplify(m, resolution, reduction_factor, max_error));
   if (m->simplified) {
     IGN_REQUIRE(reduction_factor == m->simp_factor && max_error == m->simp_max_error, IGN_ERR_INVALID,
                 "mesher was simplified with reduction_factor=%d max_error=%g; call mesh() again to change",
@@ -593,14 +529,14 @@ int ign_mesh_get(ign_mesher* m, uint64_t id, const float resolution[3], int redu
   *nv = v1 - v0;
   *nf = t1 - t0;
   if (*nv == 0 || vertices == nullptr || faces == nullptr) return IGN_OK;
-  scratch_reset(ctx);
-  IGN_TRY(scratch_reserve(ctx, (v1 - v0) * 12 + 4096));
-  float* d_pos = (float*)scratch_take(ctx, (v1 - v0) * 12);
+  Scratch sc(ctx);
+  IGN_TRY(sc.reserve((v1 - v0) * 12 + 4096));
+  float* d_pos = sc.take<float>((v1 - v0) * 3);
+  IGN_REQUIRE(sc.ok(), IGN_ERR_NOMEM, "scratch arena too small (mesh positions)");
   IGN_TRY(mesher_positions(m, v0, v1 - v0, resolution, voxel_centered, d_pos));
   IGN_CUDA(cudaMemcpyAsync(vertices, d_pos, (v1 - v0) * 12, cudaMemcpyDeviceToHost, ctx->stream));
   IGN_CUDA(cudaMemcpyAsync(faces, m->d_faces + 3 * t0, (t1 - t0) * 12, cudaMemcpyDeviceToHost, ctx->stream));
   IGN_CUDA(cudaStreamSynchronize(ctx->stream));
-  scratch_reset(ctx);
   return IGN_OK;
 }
 
@@ -620,14 +556,14 @@ int ign_mesh_export(ign_mesher* m, const float resolution[3], int voxel_centered
   vert_offsets[j] = m->U;
   face_offsets[j] = m->T;
   if (m->U == 0 || vertices == nullptr || faces == nullptr) return IGN_OK;
-  scratch_reset(ctx);
-  IGN_TRY(scratch_reserve(ctx, m->U * 12 + 4096));
-  float* d_pos = (float*)scratch_take(ctx, m->U * 12);
+  Scratch sc(ctx);
+  IGN_TRY(sc.reserve(m->U * 12 + 4096));
+  float* d_pos = sc.take<float>(m->U * 3);
+  IGN_REQUIRE(sc.ok(), IGN_ERR_NOMEM, "scratch arena too small (mesh positions)");
   IGN_TRY(mesher_positions(m, 0, m->U, resolution, voxel_centered, d_pos));
   IGN_TRY(d2h_by_kernel(ctx, vertices, d_pos, m->U * 12));
   IGN_TRY(d2h_by_kernel(ctx, faces, m->d_faces, m->T * 12));
   IGN_CUDA(cudaStreamSynchronize(ctx->stream));
-  scratch_reset(ctx);
   return IGN_OK;
 }
 

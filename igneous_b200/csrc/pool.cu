@@ -471,11 +471,19 @@ static int mode_pyramid(ign_ctx* ctx, const T* in, uint64_t sx, uint64_t sy, uin
   return IGN_OK;
 }
 
+// worst-case scratch needed by the averaging generic path
+static size_t avg_scratch_bytes(uint64_t sx, uint64_t sy, uint64_t nz) {
+  const uint64_t ox = (sx + 1) >> 1, oy = (sy + 1) >> 1;
+  return align_up(ox * oy * nz * 8, 256) * 5 / 4 + 4096;
+}
+
 // A: accumulator type wide enough for 256 * max(T)
 template <typename T, typename A>
 static int avg_pyramid(ign_ctx* ctx, const T* in, uint64_t sx, uint64_t sy, uint64_t nz,
                        int num_mips, int rounding, void* const* outs) {
   constexpr int VEC = 16 / (int)sizeof(T);
+  Scratch sc(ctx);
+  IGN_TRY(sc.reserve(avg_scratch_bytes(sx, sy, nz)));
   const T* cur = in;
   int m = 0;
   while (m < num_mips) {
@@ -508,12 +516,12 @@ static int avg_pyramid(ign_ctx* ctx, const T* in, uint64_t sx, uint64_t sy, uint
       // level by level with explicit accumulator arrays (ping-pong in scratch)
       const uint64_t ox1 = (sx + 1) >> 1, oy1 = (sy + 1) >> 1;
       const size_t acc_bytes = align_up(ox1 * oy1 * nz * sizeof(A), 256);
-      const size_t keep = ctx->scratch_used;
+      sc.rewind();
       A* acc[2] = {nullptr, nullptr};
       if (g > 1) {
-        acc[0] = (A*)scratch_take(ctx, acc_bytes);
-        acc[1] = (A*)scratch_take(ctx, acc_bytes / 4 + 256);
-        IGN_REQUIRE(acc[0] && acc[1], IGN_ERR_NOMEM, "scratch arena too small for averaging accumulators");
+        acc[0] = (A*)sc.take(acc_bytes);
+        acc[1] = (A*)sc.take(acc_bytes / 4 + 256);
+        IGN_REQUIRE(sc.ok(), IGN_ERR_NOMEM, "scratch arena too small for averaging accumulators");
       }
       for (int k = 0; k < g; k++) {
         const uint64_t ox = (sx + 1) >> 1, oy = (sy + 1) >> 1, total = ox * oy * nz;
@@ -527,7 +535,6 @@ static int avg_pyramid(ign_ctx* ctx, const T* in, uint64_t sx, uint64_t sy, uint
         sx = ox;
         sy = oy;
       }
-      ctx->scratch_used = keep;
     }
     m += g;
     cur = (const T*)outs[m - 1];
@@ -547,12 +554,6 @@ static int avg_f32_pyramid(ign_ctx* ctx, const float* in, uint64_t sx, uint64_t 
     sy = oy;
   }
   return IGN_OK;
-}
-
-// worst-case scratch needed by the averaging generic path
-static size_t avg_scratch_bytes(uint64_t sx, uint64_t sy, uint64_t nz) {
-  const uint64_t ox = (sx + 1) >> 1, oy = (sy + 1) >> 1;
-  return align_up(ox * oy * nz * 8, 256) * 5 / 4 + 4096;
 }
 
 static int check_pool_args(const void* in, int dtype, uint64_t sx, uint64_t sy, uint64_t nz,
@@ -612,6 +613,21 @@ static int select_pyramid(ign_ctx* ctx, const void* in, uint64_t sx, uint64_t sy
 
 using namespace ign;
 
+// host buffers: stage `in` and one output slot per mip, run the _dev function, copy the mips back
+template <typename Run>
+static int pool_host(ign_ctx* ctx, const void* in, uint64_t in_bytes, const uint64_t* out_bytes, int num_mips,
+                     void* const* outs, const Run& run) {
+  Staging st(ctx);
+  void* d_in;
+  void* d_out[32];
+  st.add(&d_in, in_bytes, in);
+  for (int m = 0; m < num_mips; m++) st.add(&d_out[m], out_bytes[m]);
+  IGN_TRY(st.stage());
+  IGN_TRY(run(d_in, d_out));
+  for (int m = 0; m < num_mips; m++) IGN_TRY(st.back(outs[m], d_out[m], out_bytes[m]));
+  return st.sync();
+}
+
 extern "C" {
 
 int ign_pool_mode_2x2x1_dev(ign_ctx* ctx, const void* in, int dtype, uint64_t sx, uint64_t sy,
@@ -634,10 +650,6 @@ int ign_pool_avg_2x2x1_dev(ign_ctx* ctx, const void* in, int dtype, uint64_t sx,
   IGN_TRY(activate(ctx));
   IGN_TRY(check_pool_args(in, dtype, sx, sy, sz, num_mips, outs));
   IGN_REQUIRE(rounding >= 0 && rounding <= 2, IGN_ERR_INVALID, "bad rounding mode %d", rounding);
-  if (dtype != IGN_F32) {
-    // the generic path may need accumulators: only reserve when this call owns the arena
-    if (ctx->scratch_used == 0) IGN_TRY(scratch_reserve(ctx, avg_scratch_bytes(sx, sy, sz)));
-  }
   switch (dtype) {
     case IGN_U8: return avg_pyramid<uint8_t, uint32_t>(ctx, (const uint8_t*)in, sx, sy, sz, num_mips, rounding, outs);
     case IGN_U16: return avg_pyramid<uint16_t, uint32_t>(ctx, (const uint16_t*)in, sx, sy, sz, num_mips, rounding, outs);
@@ -675,73 +687,44 @@ int ign_pool_select(ign_ctx* ctx, const void* in, int dtype, uint64_t sx, uint64
   IGN_REQUIRE(fx >= 1 && fx <= 2 && fy >= 1 && fy <= 2 && fz >= 1 && fz <= 2, IGN_ERR_UNSUPPORTED,
               "pooling factors must be 1 or 2 per axis (got %u,%u,%u)", fx, fy, fz);
   const size_t es = dtype_size(dtype);
-  size_t total = align_up(sx * sy * sz * es, 256);
-  size_t ob[32];
+  uint64_t ob[32];
   uint64_t x = sx, y = sy, z = sz;
   for (int m = 0; m < num_mips; m++) {
     x = (x + fx - 1) / fx; y = (y + fy - 1) / fy; z = (z + fz - 1) / fz;
     ob[m] = x * y * z * es;
-    total += align_up(ob[m], 256);
   }
-  scratch_reset(ctx);
-  IGN_TRY(scratch_reserve(ctx, total + 4096));
-  void* d_in = scratch_take(ctx, sx * sy * sz * es);
-  void* d_out[32];
-  for (int m = 0; m < num_mips; m++) d_out[m] = scratch_take(ctx, ob[m]);
-  IGN_CUDA(cudaMemcpyAsync(d_in, in, sx * sy * sz * es, cudaMemcpyHostToDevice, ctx->stream));
-  int rc = ign_pool_select_dev(ctx, d_in, dtype, sx, sy, sz, fx, fy, fz, num_mips, op, d_out);
-  if (rc == IGN_OK) {
-    for (int m = 0; m < num_mips; m++)
-      IGN_CUDA(cudaMemcpyAsync(outs[m], d_out[m], ob[m], cudaMemcpyDeviceToHost, ctx->stream));
-    IGN_CUDA(cudaStreamSynchronize(ctx->stream));
-  }
-  scratch_reset(ctx);
-  return rc;
+  return pool_host(ctx, in, sx * sy * sz * es, ob, num_mips, outs, [&](const void* d_in, void* const* d_out) {
+    return ign_pool_select_dev(ctx, d_in, dtype, sx, sy, sz, fx, fy, fz, num_mips, op, d_out);
+  });
 }
 
-static int pool_host(ign_ctx* ctx, bool mode, const void* in, int dtype, uint64_t sx, uint64_t sy,
-                     uint64_t sz, int num_mips, int flag, void* const* outs) {
+// 2x2x1 pyramids: every mip halves x and y
+static int pool_2x2x1_host(ign_ctx* ctx, bool mode, const void* in, int dtype, uint64_t sx, uint64_t sy,
+                           uint64_t sz, int num_mips, int flag, void* const* outs) {
   IGN_TRY(activate(ctx));
   IGN_TRY(check_pool_args(in, dtype, sx, sy, sz, num_mips, outs));
   const size_t es = dtype_size(dtype);
-  const size_t in_bytes = sx * sy * sz * es;
-  size_t total = align_up(in_bytes, 256);
+  uint64_t ob[32];
   uint64_t x = sx, y = sy;
-  size_t out_bytes[32];
   for (int m = 0; m < num_mips; m++) {
     x = (x + 1) >> 1;
     y = (y + 1) >> 1;
-    out_bytes[m] = x * y * sz * es;
-    total += align_up(out_bytes[m], 256);
+    ob[m] = x * y * sz * es;
   }
-  total += avg_scratch_bytes(sx, sy, sz);
-  scratch_reset(ctx);
-  IGN_TRY(scratch_reserve(ctx, total));
-  void* d_in = scratch_take(ctx, in_bytes);
-  void* d_out[32];
-  for (int m = 0; m < num_mips; m++) d_out[m] = scratch_take(ctx, out_bytes[m]);
-  IGN_CUDA(cudaMemcpyAsync(d_in, in, in_bytes, cudaMemcpyHostToDevice, ctx->stream));
-  int rc = mode ? ign_pool_mode_2x2x1_dev(ctx, d_in, dtype, sx, sy, sz, num_mips, flag, d_out)
+  return pool_host(ctx, in, sx * sy * sz * es, ob, num_mips, outs, [&](const void* d_in, void* const* d_out) {
+    return mode ? ign_pool_mode_2x2x1_dev(ctx, d_in, dtype, sx, sy, sz, num_mips, flag, d_out)
                 : ign_pool_avg_2x2x1_dev(ctx, d_in, dtype, sx, sy, sz, num_mips, flag, d_out);
-  if (rc != IGN_OK) {
-    scratch_reset(ctx);
-    return rc;
-  }
-  for (int m = 0; m < num_mips; m++)
-    IGN_CUDA(cudaMemcpyAsync(outs[m], d_out[m], out_bytes[m], cudaMemcpyDeviceToHost, ctx->stream));
-  IGN_CUDA(cudaStreamSynchronize(ctx->stream));
-  scratch_reset(ctx);
-  return IGN_OK;
+  });
 }
 
 int ign_pool_mode_2x2x1(ign_ctx* ctx, const void* in, int dtype, uint64_t sx, uint64_t sy,
                         uint64_t sz, int num_mips, int sparse, void* const* outs) {
-  return pool_host(ctx, true, in, dtype, sx, sy, sz, num_mips, sparse, outs);
+  return pool_2x2x1_host(ctx, true, in, dtype, sx, sy, sz, num_mips, sparse, outs);
 }
 
 int ign_pool_avg_2x2x1(ign_ctx* ctx, const void* in, int dtype, uint64_t sx, uint64_t sy,
                        uint64_t sz, int num_mips, int rounding, void* const* outs) {
-  return pool_host(ctx, false, in, dtype, sx, sy, sz, num_mips, rounding, outs);
+  return pool_2x2x1_host(ctx, false, in, dtype, sx, sy, sz, num_mips, rounding, outs);
 }
 
 }  // extern "C"

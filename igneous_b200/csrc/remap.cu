@@ -266,12 +266,12 @@ static uint32_t pow2_at_least(uint64_t v) {
   return (uint32_t)c;
 }
 
-static int table_alloc(ign_ctx* ctx, uint32_t cap, uint64_t val_init_byte, HashTable& t,
+static int table_alloc(ign_ctx* ctx, Scratch& sc, uint32_t cap, uint64_t val_init_byte, HashTable& t,
                        uint32_t** counters) {
-  t.keys = (uint64_t*)scratch_take(ctx, (size_t)cap * 8);
-  t.vals = (uint64_t*)scratch_take(ctx, ((size_t)cap + 1) * 8);
-  *counters = (uint32_t*)scratch_take(ctx, 256);
-  IGN_REQUIRE(t.keys && t.vals && *counters, IGN_ERR_NOMEM, "scratch arena too small for hash table");
+  t.keys = sc.take<uint64_t>(cap);
+  t.vals = sc.take<uint64_t>((size_t)cap + 1);
+  *counters = sc.take<uint32_t>(64);
+  IGN_REQUIRE(sc.ok(), IGN_ERR_NOMEM, "scratch arena too small for hash table");
   t.side = *counters + 2;
   t.mask = cap - 1;
   IGN_CUDA(cudaMemsetAsync(t.keys, 0xFF, (size_t)cap * 8, ctx->stream));
@@ -305,21 +305,19 @@ static size_t sort_tmp_bytes_u64(uint32_t n) {
 }
 
 // Builds the first-appearance table for `in` and assigns ids; leaves table in t.
-// Retries with a larger table on overflow.  Caller owns the arena bump pointer.
-static int renumber_table(ign_ctx* ctx, const void* in, int dtype, uint64_t n, HashTable& t,
+// Retries with a larger table on overflow.  The table lives in the caller's scope `sc`.
+static int renumber_table(ign_ctx* ctx, Scratch& sc, const void* in, int dtype, uint64_t n, HashTable& t,
                           uint32_t** counters_out, uint64_t* uniq_dev, uint64_t uniq_cap,
                           uint64_t* k_out) {
   IGN_REQUIRE(n < 0xFFFFFFFFull, IGN_ERR_OVERFLOW, "renumber: more than 2^32 elements");
-  const bool own = (ctx->scratch_used == 0);
   uint32_t cap = pow2_at_least(n < (1u << 19) ? 2 * n + 16 : (1u << 20));
   const uint32_t cap_max = pow2_at_least(2 * n + 16);
-  const size_t keep = ctx->scratch_used;
   while (true) {
-    ctx->scratch_used = keep;
+    sc.rewind();
     const size_t need = (size_t)cap * 16 + (size_t)cap * (8 + 4 + 8 + 4) + sort_tmp_bytes_u64(cap) + 8192;
-    if (own) IGN_TRY(scratch_reserve(ctx, need));
+    IGN_TRY(sc.reserve(need));
     uint32_t* counters;
-    IGN_TRY(table_alloc(ctx, cap, 0xFF, t, &counters));
+    IGN_TRY(table_alloc(ctx, sc, cap, 0xFF, t, &counters));
 #define RUN_FIRST(T, dummy) IGN_LAUNCH(ctx, (k_first_index<T>), blocks_for(n, 256), 256, 0, (const T*)in, n, t, counters)
     DISPATCH_UINT(dtype, RUN_FIRST, 0)
 #undef RUN_FIRST
@@ -331,13 +329,13 @@ static int renumber_table(ign_ctx* ctx, const void* in, int dtype, uint64_t n, H
       continue;
     }
     const uint32_t total = h[0];
-    uint64_t* firsts = (uint64_t*)scratch_take(ctx, (size_t)total * 8 + 8);
-    uint32_t* slots = (uint32_t*)scratch_take(ctx, (size_t)total * 4 + 4);
-    uint64_t* firsts_s = (uint64_t*)scratch_take(ctx, (size_t)total * 8 + 8);
-    uint32_t* slots_s = (uint32_t*)scratch_take(ctx, (size_t)total * 4 + 4);
+    uint64_t* firsts = sc.take<uint64_t>((size_t)total + 1);
+    uint32_t* slots = sc.take<uint32_t>((size_t)total + 1);
+    uint64_t* firsts_s = sc.take<uint64_t>((size_t)total + 1);
+    uint32_t* slots_s = sc.take<uint32_t>((size_t)total + 1);
     size_t tmp_bytes = sort_tmp_bytes_u64(total ? total : 1);
-    void* tmp = scratch_take(ctx, tmp_bytes);
-    IGN_REQUIRE(firsts && slots && firsts_s && slots_s && tmp, IGN_ERR_NOMEM, "scratch arena too small (renumber)");
+    void* tmp = sc.take(tmp_bytes);
+    IGN_REQUIRE(sc.ok(), IGN_ERR_NOMEM, "scratch arena too small (renumber)");
     uint64_t k = 0;
     if (total > 0) {
       IGN_LAUNCH(ctx, k_compact_slots, blocks_for((uint64_t)cap + 1, 256), 256, 0, t, firsts, slots, counters);
@@ -389,17 +387,14 @@ int ign_renumber_dev(ign_ctx* ctx, const void* in, int dtype, uint64_t n, uint32
   IGN_REQUIRE(in && out && k, IGN_ERR_INVALID, "null argument");
   *k = 0;
   if (n == 0) return IGN_OK;
-  const size_t keep = ctx->scratch_used;
+  Scratch sc(ctx);
   HashTable t;
   uint32_t* counters;
-  int rc = renumber_table(ctx, in, dtype, n, t, &counters, uniq_dev, uniq_capacity, k);
-  if (rc == IGN_OK) {
+  IGN_TRY(renumber_table(ctx, sc, in, dtype, n, t, &counters, uniq_dev, uniq_capacity, k));
 #define RUN_GATHER(T, dummy) IGN_LAUNCH(ctx, (k_gather<T, uint32_t>), blocks_for(n, 256), 256, 0, (const T*)in, n, t, out)
-    DISPATCH_UINT(dtype, RUN_GATHER, 0)
+  DISPATCH_UINT(dtype, RUN_GATHER, 0)
 #undef RUN_GATHER
-  }
-  ctx->scratch_used = keep;
-  return rc;
+  return IGN_OK;
 }
 
 int ign_renumber(ign_ctx* ctx, const void* in, int dtype, uint64_t n, uint32_t* out, uint64_t* uniq,
@@ -411,25 +406,16 @@ int ign_renumber(ign_ctx* ctx, const void* in, int dtype, uint64_t n, uint32_t* 
   const int es = dtype_size(dtype);
   IGN_REQUIRE(es > 0 && dtype != IGN_F32, IGN_ERR_UNSUPPORTED, "unsupported dtype %d", dtype);
   IGN_REQUIRE(n < 0xFFFFFFFFull, IGN_ERR_OVERFLOW, "renumber: more than 2^32 elements");
-  scratch_reset(ctx);
-  const uint32_t cap_max = pow2_at_least(2 * n + 16);
-  const size_t table = (size_t)cap_max * 16 + (size_t)cap_max * 24 + sort_tmp_bytes_u64(cap_max) + 16384;
-  IGN_TRY(scratch_reserve(ctx, align_up(n * es, 256) + align_up(n * 4, 256) + align_up(uniq_capacity * 8, 256) + table));
-  void* d_in = scratch_take(ctx, n * es);
-  uint32_t* d_out = (uint32_t*)scratch_take(ctx, n * 4);
-  uint64_t* d_uniq = uniq_capacity ? (uint64_t*)scratch_take(ctx, uniq_capacity * 8) : nullptr;
-  IGN_CUDA(cudaMemcpyAsync(d_in, in, n * es, cudaMemcpyHostToDevice, ctx->stream));
-  int rc = ign_renumber_dev(ctx, d_in, dtype, n, d_out, d_uniq, uniq_capacity, k);
-  if (rc == IGN_OK) {
-    IGN_CUDA(cudaMemcpyAsync(out, d_out, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
-    if (uniq && d_uniq) {
-      const uint64_t m = (*k < uniq_capacity) ? *k : uniq_capacity;
-      IGN_CUDA(cudaMemcpyAsync(uniq, d_uniq, m * 8, cudaMemcpyDeviceToHost, ctx->stream));
-    }
-    IGN_CUDA(cudaStreamSynchronize(ctx->stream));
-  }
-  scratch_reset(ctx);
-  return rc;
+  Staging st(ctx);
+  void *d_in, *d_out, *d_uniq;
+  st.add(&d_in, n * es, in);
+  st.add(&d_out, n * 4);
+  st.add(&d_uniq, uniq_capacity * 8);
+  IGN_TRY(st.stage());
+  IGN_TRY(ign_renumber_dev(ctx, d_in, dtype, n, (uint32_t*)d_out, (uint64_t*)d_uniq, uniq_capacity, k));
+  IGN_TRY(st.back(out, d_out, n * 4));
+  if (uniq) IGN_TRY(st.back(uniq, d_uniq, (*k < uniq_capacity ? *k : uniq_capacity) * 8));
+  return st.sync();
 }
 
 // keys/vals are HOST arrays (the table is small); arr is a DEVICE array
@@ -438,17 +424,16 @@ int ign_remap_dev(ign_ctx* ctx, void* arr, int dtype, uint64_t n, const uint64_t
   IGN_TRY(activate(ctx));
   IGN_REQUIRE(arr && (n_keys == 0 || (keys_host && vals_host)), IGN_ERR_INVALID, "null argument");
   if (n == 0) return IGN_OK;
-  const bool own = (ctx->scratch_used == 0);
-  const size_t keep = ctx->scratch_used;
+  Scratch sc(ctx);
   const uint32_t cap = pow2_at_least(2 * n_keys + 16);
-  if (own) IGN_TRY(scratch_reserve(ctx, (size_t)cap * 16 + n_keys * 16 + 8192));
+  IGN_TRY(sc.reserve((size_t)cap * 16 + n_keys * 16 + 8192));
   HashTable t;
   uint32_t* counters;
-  IGN_TRY(table_alloc(ctx, cap, 0, t, &counters));
-  uint64_t* dk = (uint64_t*)scratch_take(ctx, n_keys * 8 + 8);
-  uint64_t* dv = (uint64_t*)scratch_take(ctx, n_keys * 8 + 8);
-  uint64_t* dmiss = (uint64_t*)scratch_take(ctx, 8);
-  IGN_REQUIRE(dk && dv && dmiss, IGN_ERR_NOMEM, "scratch arena too small (remap)");
+  IGN_TRY(table_alloc(ctx, sc, cap, 0, t, &counters));
+  uint64_t* dk = sc.take<uint64_t>(n_keys + 1);
+  uint64_t* dv = sc.take<uint64_t>(n_keys + 1);
+  uint64_t* dmiss = sc.take<uint64_t>(1);
+  IGN_REQUIRE(sc.ok(), IGN_ERR_NOMEM, "scratch arena too small (remap)");
   if (n_keys) {
     IGN_CUDA(cudaMemcpyAsync(dk, keys_host, n_keys * 8, cudaMemcpyHostToDevice, ctx->stream));
     IGN_CUDA(cudaMemcpyAsync(dv, vals_host, n_keys * 8, cudaMemcpyHostToDevice, ctx->stream));
@@ -459,15 +444,13 @@ int ign_remap_dev(ign_ctx* ctx, void* arr, int dtype, uint64_t n, const uint64_t
 #undef RUN_REMAP
   uint32_t h[8];
   IGN_TRY(read_counters(ctx, counters, h));
-  int rc = IGN_OK;
   if (h[5] != 0) {
     uint64_t miss = 0;
     IGN_CUDA(cudaMemcpy(&miss, dmiss, 8, cudaMemcpyDeviceToHost));
     set_error("%llu", (unsigned long long)miss);  // KeyError(label), as fastremap.remap
-    rc = IGN_ERR_KEY;
+    return IGN_ERR_KEY;
   }
-  ctx->scratch_used = keep;
-  return rc;
+  return IGN_OK;
 }
 
 int ign_remap(ign_ctx* ctx, void* arr, int dtype, uint64_t n, const uint64_t* keys,
@@ -477,18 +460,13 @@ int ign_remap(ign_ctx* ctx, void* arr, int dtype, uint64_t n, const uint64_t* ke
   if (n == 0) return IGN_OK;
   const int es = dtype_size(dtype);
   IGN_REQUIRE(es > 0 && dtype != IGN_F32, IGN_ERR_UNSUPPORTED, "unsupported dtype %d", dtype);
-  scratch_reset(ctx);
-  const uint32_t cap = pow2_at_least(2 * n_keys + 16);
-  IGN_TRY(scratch_reserve(ctx, align_up(n * es, 256) + (size_t)cap * 16 + n_keys * 16 + 16384));
-  void* d = scratch_take(ctx, n * es);
-  IGN_CUDA(cudaMemcpyAsync(d, arr, n * es, cudaMemcpyHostToDevice, ctx->stream));
-  int rc = ign_remap_dev(ctx, d, dtype, n, keys, vals, n_keys, preserve_missing);
-  if (rc == IGN_OK) {
-    IGN_CUDA(cudaMemcpyAsync(arr, d, n * es, cudaMemcpyDeviceToHost, ctx->stream));
-    IGN_CUDA(cudaStreamSynchronize(ctx->stream));
-  }
-  scratch_reset(ctx);
-  return rc;
+  Staging st(ctx);
+  void* d;
+  st.add(&d, n * es, arr);
+  IGN_TRY(st.stage());
+  IGN_TRY(ign_remap_dev(ctx, d, dtype, n, keys, vals, n_keys, preserve_missing));
+  IGN_TRY(st.back(arr, d, n * es));
+  return st.sync();
 }
 
 int ign_mask(ign_ctx* ctx, void* arr, int dtype, uint64_t n, const uint64_t* labels,
@@ -498,16 +476,18 @@ int ign_mask(ign_ctx* ctx, void* arr, int dtype, uint64_t n, const uint64_t* lab
   if (n == 0) return IGN_OK;
   const int es = dtype_size(dtype);
   IGN_REQUIRE(es > 0 && dtype != IGN_F32, IGN_ERR_UNSUPPORTED, "unsupported dtype %d", dtype);
-  scratch_reset(ctx);
+  Staging st(ctx);
+  void* d;
+  st.add(&d, n * es, arr);
+  IGN_TRY(st.stage());
+  Scratch sc(ctx);
   const uint32_t cap = pow2_at_least(2 * n_labels + 16);
-  IGN_TRY(scratch_reserve(ctx, align_up(n * es, 256) + (size_t)cap * 16 + n_labels * 8 + 16384));
-  void* d = scratch_take(ctx, n * es);
+  IGN_TRY(sc.reserve((size_t)cap * 16 + n_labels * 8 + 16384));
   HashTable t;
   uint32_t* counters;
-  IGN_TRY(table_alloc(ctx, cap, 0, t, &counters));
-  uint64_t* dk = (uint64_t*)scratch_take(ctx, n_labels * 8 + 8);
-  IGN_REQUIRE(d && dk, IGN_ERR_NOMEM, "scratch arena too small (mask)");
-  IGN_CUDA(cudaMemcpyAsync(d, arr, n * es, cudaMemcpyHostToDevice, ctx->stream));
+  IGN_TRY(table_alloc(ctx, sc, cap, 0, t, &counters));
+  uint64_t* dk = sc.take<uint64_t>(n_labels + 1);
+  IGN_REQUIRE(sc.ok(), IGN_ERR_NOMEM, "scratch arena too small (mask)");
   if (n_labels) {
     IGN_CUDA(cudaMemcpyAsync(dk, labels, n_labels * 8, cudaMemcpyHostToDevice, ctx->stream));
     IGN_LAUNCH(ctx, k_table_build, blocks_for(n_labels, 256), 256, 0, dk, (const uint64_t*)nullptr, n_labels, t, counters);
@@ -515,10 +495,8 @@ int ign_mask(ign_ctx* ctx, void* arr, int dtype, uint64_t n, const uint64_t* lab
 #define RUN_MASK(T, dummy) IGN_LAUNCH(ctx, (k_mask<T>), blocks_for(n, 256), 256, 0, (T*)d, n, t, except, (T)value)
   DISPATCH_UINT(dtype, RUN_MASK, 0)
 #undef RUN_MASK
-  IGN_CUDA(cudaMemcpyAsync(arr, d, n * es, cudaMemcpyDeviceToHost, ctx->stream));
-  IGN_CUDA(cudaStreamSynchronize(ctx->stream));
-  scratch_reset(ctx);
-  return IGN_OK;
+  IGN_TRY(st.back(arr, d, n * es));
+  return st.sync();
 }
 
 int ign_unique(ign_ctx* ctx, const void* in, int dtype, uint64_t n, uint64_t* uniq, uint64_t* counts,
@@ -530,17 +508,19 @@ int ign_unique(ign_ctx* ctx, const void* in, int dtype, uint64_t n, uint64_t* un
   const int es = dtype_size(dtype);
   IGN_REQUIRE(es > 0 && dtype != IGN_F32, IGN_ERR_UNSUPPORTED, "unsupported dtype %d", dtype);
   IGN_REQUIRE(n < 0xFFFFFFFFull, IGN_ERR_OVERFLOW, "unique: more than 2^32 elements");
-  scratch_reset(ctx);
+  Staging st(ctx);
+  void* d_in;
+  st.add(&d_in, n * es, in);
+  IGN_TRY(st.stage());
+  Scratch sc(ctx);
   uint32_t cap = pow2_at_least(n < (1u << 19) ? 2 * n + 16 : (1u << 20));
   const uint32_t cap_max = pow2_at_least(2 * n + 16);
   while (true) {
-    scratch_reset(ctx);
-    IGN_TRY(scratch_reserve(ctx, align_up(n * es, 256) + (size_t)cap * 16 + (size_t)cap * 32 + sort_tmp_bytes_u64(cap) + 16384));
-    void* d_in = scratch_take(ctx, n * es);
+    sc.rewind();
+    IGN_TRY(sc.reserve((size_t)cap * 16 + (size_t)cap * 32 + sort_tmp_bytes_u64(cap) + 16384));
     HashTable t;
     uint32_t* counters;
-    IGN_TRY(table_alloc(ctx, cap, 0, t, &counters));
-    IGN_CUDA(cudaMemcpyAsync(d_in, in, n * es, cudaMemcpyHostToDevice, ctx->stream));
+    IGN_TRY(table_alloc(ctx, sc, cap, 0, t, &counters));
 #define RUN_COUNT(T, dummy) IGN_LAUNCH(ctx, (k_count<T>), blocks_for(n, 256), 256, 0, (const T*)d_in, n, t, counters)
     DISPATCH_UINT(dtype, RUN_COUNT, 0)
 #undef RUN_COUNT
@@ -554,22 +534,21 @@ int ign_unique(ign_ctx* ctx, const void* in, int dtype, uint64_t n, uint64_t* un
     const uint32_t total = h[0];
     *k = total;
     if (uniq != nullptr && total > 0) {
-      uint64_t* ck = (uint64_t*)scratch_take(ctx, (size_t)total * 8);
-      uint64_t* cv = (uint64_t*)scratch_take(ctx, (size_t)total * 8);
-      uint64_t* sk = (uint64_t*)scratch_take(ctx, (size_t)total * 8);
-      uint64_t* sv = (uint64_t*)scratch_take(ctx, (size_t)total * 8);
+      uint64_t* ck = sc.take<uint64_t>(total);
+      uint64_t* cv = sc.take<uint64_t>(total);
+      uint64_t* sk = sc.take<uint64_t>(total);
+      uint64_t* sv = sc.take<uint64_t>(total);
       size_t tmp_bytes = sort_tmp_bytes_u64(total);
-      void* tmp = scratch_take(ctx, tmp_bytes);
-      IGN_REQUIRE(ck && cv && sk && sv && tmp, IGN_ERR_NOMEM, "scratch arena too small (unique)");
+      void* tmp = sc.take(tmp_bytes);
+      IGN_REQUIRE(sc.ok(), IGN_ERR_NOMEM, "scratch arena too small (unique)");
       IGN_LAUNCH(ctx, k_compact_kv, blocks_for((uint64_t)cap + 1, 256), 256, 0, t, ck, cv, counters);
       IGN_CUDA(cub::DeviceRadixSort::SortPairs(tmp, tmp_bytes, ck, sk, cv, sv, (int)total, 0, 64, ctx->stream));
       ctx->launches += 2;
       const uint64_t m = total < capacity ? total : capacity;
-      IGN_CUDA(cudaMemcpyAsync(uniq, sk, m * 8, cudaMemcpyDeviceToHost, ctx->stream));
-      if (counts) IGN_CUDA(cudaMemcpyAsync(counts, sv, m * 8, cudaMemcpyDeviceToHost, ctx->stream));
-      IGN_CUDA(cudaStreamSynchronize(ctx->stream));
+      IGN_TRY(st.back(uniq, sk, m * 8));
+      if (counts) IGN_TRY(st.back(counts, sv, m * 8));
+      IGN_TRY(st.sync());
     }
-    scratch_reset(ctx);
     return IGN_OK;
   }
 }
@@ -584,24 +563,25 @@ int ign_inverse_component_map(ign_ctx* ctx, const void* parents, const void* com
   const int es = dtype_size(dtype);
   IGN_REQUIRE(es > 0 && dtype != IGN_F32, IGN_ERR_UNSUPPORTED, "unsupported dtype %d", dtype);
   IGN_REQUIRE(n < 0x7FFFFFFFull, IGN_ERR_OVERFLOW, "inverse_component_map: too many elements");
-  scratch_reset(ctx);
+  Staging st(ctx);
+  void *dp, *dc;
+  st.add(&dp, n * es, parents);
+  st.add(&dc, n * es, components);
+  IGN_TRY(st.stage());
+  Scratch sc(ctx);
   size_t scan_bytes = 0;
   cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, (const uint32_t*)nullptr, (uint32_t*)nullptr, (int)n);
   const size_t tmp_bytes = sort_tmp_bytes_u64((uint32_t)n) + scan_bytes;
-  IGN_TRY(scratch_reserve(ctx, 2 * align_up(n * es, 256) + 4 * align_up(n * 8, 256) + 2 * align_up(n * 4, 256) + align_up(n * 16, 256) + tmp_bytes + 16384));
-  void* dp = scratch_take(ctx, n * es);
-  void* dc = scratch_take(ctx, n * es);
-  uint64_t* p0 = (uint64_t*)scratch_take(ctx, n * 8);
-  uint64_t* c0 = (uint64_t*)scratch_take(ctx, n * 8);
-  uint64_t* p1 = (uint64_t*)scratch_take(ctx, n * 8);
-  uint64_t* c1 = (uint64_t*)scratch_take(ctx, n * 8);
-  uint32_t* flags = (uint32_t*)scratch_take(ctx, n * 4);
-  uint32_t* pos = (uint32_t*)scratch_take(ctx, n * 4 + 4);
-  uint64_t* dout = (uint64_t*)scratch_take(ctx, n * 16);
-  void* tmp = scratch_take(ctx, tmp_bytes);
-  IGN_REQUIRE(dp && dc && p0 && c0 && p1 && c1 && flags && pos && dout && tmp, IGN_ERR_NOMEM, "scratch arena too small (inverse_component_map)");
-  IGN_CUDA(cudaMemcpyAsync(dp, parents, n * es, cudaMemcpyHostToDevice, ctx->stream));
-  IGN_CUDA(cudaMemcpyAsync(dc, components, n * es, cudaMemcpyHostToDevice, ctx->stream));
+  IGN_TRY(sc.reserve(4 * align_up(n * 8, 256) + 2 * align_up(n * 4, 256) + align_up(n * 16, 256) + tmp_bytes + 16384));
+  uint64_t* p0 = sc.take<uint64_t>(n);
+  uint64_t* c0 = sc.take<uint64_t>(n);
+  uint64_t* p1 = sc.take<uint64_t>(n);
+  uint64_t* c1 = sc.take<uint64_t>(n);
+  uint32_t* flags = sc.take<uint32_t>(n);
+  uint32_t* pos = sc.take<uint32_t>(n + 1);
+  uint64_t* dout = sc.take<uint64_t>(2 * n);
+  void* tmp = sc.take(tmp_bytes);
+  IGN_REQUIRE(sc.ok(), IGN_ERR_NOMEM, "scratch arena too small (inverse_component_map)");
 #define RUN_WIDEN(T, dummy) IGN_LAUNCH(ctx, (k_widen_pairs<T>), blocks_for(n, 256), 256, 0, (const T*)dp, (const T*)dc, n, p0, c0)
   DISPATCH_UINT(dtype, RUN_WIDEN, 0)
 #undef RUN_WIDEN
@@ -626,7 +606,6 @@ int ign_inverse_component_map(ign_ctx* ctx, const void* parents, const void* com
     const uint64_t m = total < capacity ? total : capacity;
     IGN_CUDA(cudaMemcpy(pairs, dout, m * 16, cudaMemcpyDeviceToHost));
   }
-  scratch_reset(ctx);
   return IGN_OK;
 }
 

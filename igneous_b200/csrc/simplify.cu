@@ -1180,7 +1180,8 @@ extern "C" int ign_mesh_simplify(ign_mesher* m, const float resolution[3], int r
     m->d_pos_f = nullptr;
     return IGN_OK;
   }
-  IGN_REQUIRE(ctx->scratch_used == 0, IGN_ERR_INVALID, "ign_mesh_simplify must own the scratch arena");
+  Scratch sc(ctx);
+  IGN_REQUIRE(sc.owner(), IGN_ERR_INVALID, "ign_mesh_simplify must own the scratch arena");
 
   size_t sortb = 0, scanb = 0;
   cub::DeviceRadixSort::SortPairs(nullptr, sortb, (const uint32_t*)nullptr, (uint32_t*)nullptr,
@@ -1195,74 +1196,43 @@ extern "C" int ign_mesh_simplify(ign_mesher* m, const float resolution[3], int r
                       2 * align_up(3 * T * 4, 256) + 2 * align_up(T * 4, 256) + 2 * align_up(U * 4, 256) + tmpb +
                       align_up((size_t)ctx->sm_count * 4 * SL_WCAP * 2 * S_MAXV * 4, 256) +
                       align_up((size_t)ctx->sm_count * 4 * SL_WCAP * 3 * 8, 256) + (1 << 20);
-  IGN_TRY(scratch_reserve(ctx, need));
+  IGN_TRY(sc.reserve(need));
   Simp s;
   s.U = U;
   s.T = T;
-  s.pos = (double*)scratch_take(ctx, U * 24);
-  s.Q = (double*)scratch_take(ctx, U * 80);
-  s.face = (uint32_t*)scratch_take(ctx, 3 * T * 4);
-  s.vf = (uint32_t*)scratch_take(ctx, U * S_VCAP * 4);
-  uint32_t* node_v = (uint32_t*)scratch_take(ctx, 3 * T * 4);   // reused as face scan later
-  uint32_t* node_h = (uint32_t*)scratch_take(ctx, 3 * T * 4);
-  s.flabel = (uint32_t*)scratch_take(ctx, T * 4);
-  s.falive = (uint8_t*)scratch_take(ctx, T);
-  uint8_t* fstate = (uint8_t*)scratch_take(ctx, T);
-  s.valive = (uint8_t*)scratch_take(ctx, U);
-  s.vbound = (uint8_t*)scratch_take(ctx, U);
-  uint8_t* vflag = (uint8_t*)scratch_take(ctx, U);
-  uint8_t* vlose = (uint8_t*)scratch_take(ctx, U);
-  s.vn = (uint32_t*)scratch_take(ctx, U * 4);
-  uint32_t* vscan = (uint32_t*)scratch_take(ctx, U * 4);
-  uint32_t* vflag32 = (uint32_t*)scratch_take(ctx, U * 4);
-  unsigned long long* key1 = (unsigned long long*)scratch_take(ctx, U * 8);
-  uint32_t* d_target = (uint32_t*)scratch_take(ctx, (K + 2) * 4);
-  uint32_t* d_tri_off = (uint32_t*)scratch_take(ctx, (K + 2) * 4);
-  uint32_t* d_vert_off = (uint32_t*)scratch_take(ctx, (K + 2) * 4);
-  uint32_t* d_new_tri_off = (uint32_t*)scratch_take(ctx, (K + 2) * 4);
-  uint32_t* d_new_vert_off = (uint32_t*)scratch_take(ctx, (K + 2) * 4);
-  uint32_t* d_order = (uint32_t*)scratch_take(ctx, (K + 2) * 4);
-  uint32_t* flags = (uint32_t*)scratch_take(ctx, 256);
-  float* ecost = (float*)scratch_take(ctx, 3 * T * 4);
+  s.pos = sc.take<double>(U * 3);
+  s.Q = sc.take<double>(U * 10);
+  s.face = sc.take<uint32_t>(3 * T);
+  s.vf = sc.take<uint32_t>(U * S_VCAP);
+  uint32_t* node_v = sc.take<uint32_t>(3 * T);   // reused as face scan later
+  uint32_t* node_h = sc.take<uint32_t>(3 * T);
+  s.flabel = sc.take<uint32_t>(T);
+  s.falive = sc.take<uint8_t>(T);
+  uint8_t* fstate = sc.take<uint8_t>(T);
+  s.valive = sc.take<uint8_t>(U);
+  s.vbound = sc.take<uint8_t>(U);
+  uint8_t* vflag = sc.take<uint8_t>(U);
+  uint8_t* vlose = sc.take<uint8_t>(U);
+  s.vn = sc.take<uint32_t>(U);
+  uint32_t* vscan = sc.take<uint32_t>(U);
+  uint32_t* vflag32 = sc.take<uint32_t>(U);
+  unsigned long long* key1 = sc.take<unsigned long long>(U);
+  uint32_t* d_target = sc.take<uint32_t>(K + 2);
+  uint32_t* d_tri_off = sc.take<uint32_t>(K + 2);
+  uint32_t* d_vert_off = sc.take<uint32_t>(K + 2);
+  uint32_t* d_new_tri_off = sc.take<uint32_t>(K + 2);
+  uint32_t* d_new_vert_off = sc.take<uint32_t>(K + 2);
+  uint32_t* d_order = sc.take<uint32_t>(K + 2);
+  uint32_t* flags = sc.take<uint32_t>(64);
+  float* ecost = sc.take<float>(3 * T);
   // alive lists of the global-memory class (ping-pong); the init scratch is free by then
-  uint32_t* gl_f[2] = {(uint32_t*)scratch_take(ctx, T * 4), (uint32_t*)scratch_take(ctx, T * 4)};
-  uint32_t* gl_v[2] = {(uint32_t*)scratch_take(ctx, U * 4), (uint32_t*)scratch_take(ctx, U * 4)};
-  void* tmp = scratch_take(ctx, tmpb);
-  uint32_t* sorted_v = (uint32_t*)scratch_take(ctx, 3 * T * 4);
-  uint32_t* sorted_h = (uint32_t*)scratch_take(ctx, 3 * T * 4);
-  if (!s.pos || !s.Q || !s.face || !s.vf || !node_v || !node_h || !s.flabel || !s.falive || !fstate ||
-      !s.valive || !s.vbound || !vflag || !vlose || !s.vn || !vscan || !vflag32 || !key1 || !d_target || !d_tri_off ||
-      !d_vert_off || !d_new_tri_off || !d_new_vert_off || !d_order || !flags || !ecost || !tmp || !gl_f[0] ||
-      !gl_f[1] || !gl_v[0] || !gl_v[1] ||
-      !sorted_v || !sorted_h) {
-    scratch_reset(ctx);
-    set_error("scratch arena too small (simplify: %llu faces)", (unsigned long long)T);
-    return IGN_ERR_NOMEM;
-  }
+  uint32_t* gl_f[2] = {sc.take<uint32_t>(T), sc.take<uint32_t>(T)};
+  uint32_t* gl_v[2] = {sc.take<uint32_t>(U), sc.take<uint32_t>(U)};
+  void* tmp = sc.take(tmpb);
+  uint32_t* sorted_v = sc.take<uint32_t>(3 * T);
+  uint32_t* sorted_h = sc.take<uint32_t>(3 * T);
+  IGN_REQUIRE(sc.ok(), IGN_ERR_NOMEM, "scratch arena too small (simplify: %llu faces)", (unsigned long long)T);
   s.tri_off = d_tri_off;
-  auto done = [&](int code) {
-    scratch_reset(ctx);
-    return code;
-  };
-#define S_CUDA(call)                                                                  \
-  do {                                                                                \
-    cudaError_t _e = (call);                                                          \
-    if (_e != cudaSuccess) {                                                          \
-      set_error("%s:%d: %s -> %s", __FILE__, __LINE__, #call, cudaGetErrorString(_e)); \
-      return done(IGN_ERR_CUDA);                                                      \
-    }                                                                                 \
-  } while (0)
-#define S_TRY(call)                       \
-  do {                                    \
-    const int _s = (call);                \
-    if (_s != IGN_OK) return done(_s);    \
-  } while (0)
-#define S_LAUNCH(kernel, g, b, ...)                       \
-  do {                                                    \
-    kernel<<<(g), (b), 0, ctx->stream>>>(__VA_ARGS__);    \
-    ctx->launches++;                                      \
-    S_CUDA(cudaGetLastError());                           \
-  } while (0)
 
   std::vector<uint32_t> target(K + 2, 0);
   for (uint64_t l = 1; l <= K; l++)
@@ -1274,27 +1244,27 @@ extern "C" int ign_mesh_simplify(ign_mesher* m, const float resolution[3], int r
     const uint32_t ta = m->tri_off[a + 1] - m->tri_off[a], tb = m->tri_off[b + 1] - m->tri_off[b];
     return ta != tb ? ta > tb : a < b;
   });
-  S_TRY(small_h2d(ctx, d_target, target.data(), (K + 2) * 4));
-  S_TRY(small_h2d(ctx, d_tri_off, m->tri_off.data(), (K + 2) * 4));
-  S_TRY(small_h2d(ctx, d_vert_off, m->vert_off.data(), (K + 2) * 4));
-  S_TRY(small_h2d(ctx, d_order, order.data(), K * 4));
-  S_LAUNCH(k_simp_init_verts, blocks_for(U, 256), 256, m->d_uniq_vkeys, U, (double)resolution[0],
+  IGN_TRY(small_h2d(ctx, d_target, target.data(), (K + 2) * 4));
+  IGN_TRY(small_h2d(ctx, d_tri_off, m->tri_off.data(), (K + 2) * 4));
+  IGN_TRY(small_h2d(ctx, d_vert_off, m->vert_off.data(), (K + 2) * 4));
+  IGN_TRY(small_h2d(ctx, d_order, order.data(), K * 4));
+  IGN_LAUNCH(ctx, k_simp_init_verts, blocks_for(U, 256), 256, 0, m->d_uniq_vkeys, U, (double)resolution[0],
            (double)resolution[1], (double)resolution[2], s.pos, s.valive, s.vbound, s.vn);
-  S_LAUNCH(k_simp_init_faces, blocks_for(T, 256), 256, m->d_faces, d_tri_off, d_vert_off, (uint32_t)K, T,
+  IGN_LAUNCH(ctx, k_simp_init_faces, blocks_for(T, 256), 256, 0, m->d_faces, d_tri_off, d_vert_off, (uint32_t)K, T,
            s.face, s.flabel, s.falive, node_v, node_h);
   {
     int bits = 1;
     while (bits < 32 && (1ull << bits) < U) bits++;
     size_t tb = tmpb;
-    S_CUDA(cub::DeviceRadixSort::SortPairs(tmp, tb, node_v, sorted_v, node_h, sorted_h, (int)(3 * T), 0, bits,
+    IGN_CUDA(cub::DeviceRadixSort::SortPairs(tmp, tb, node_v, sorted_v, node_h, sorted_h, (int)(3 * T), 0, bits,
                                            ctx->stream));
     ctx->launches += 3;
   }
-  S_CUDA(cudaMemsetAsync(flags, 0, 64, ctx->stream));
-  S_LAUNCH(k_simp_link, blocks_for(3 * T, 256), 256, sorted_v, sorted_h, (uint64_t)(3 * T), s.vf, s.vn,
+  IGN_CUDA(cudaMemsetAsync(flags, 0, 64, ctx->stream));
+  IGN_LAUNCH(ctx, k_simp_link, blocks_for(3 * T, 256), 256, 0, sorted_v, sorted_h, (uint64_t)(3 * T), s.vf, s.vn,
            flags + 12);
-  S_LAUNCH(k_simp_quadrics, blocks_for(U, 128), 128, s);
-  S_LAUNCH(k_simp_boundary, blocks_for(3 * T, 256), 256, s);
+  IGN_LAUNCH(ctx, k_simp_quadrics, blocks_for(U, 128), 128, 0, s);
+  IGN_LAUNCH(ctx, k_simp_boundary, blocks_for(3 * T, 256), 256, 0, s);
 
   // ---- all rounds of every label: persistent CTAs pull labels off the order list.  The kernel is
   // latency bound (barriers, dependent loads), so several CTAs per SM overlap each other's
@@ -1307,7 +1277,7 @@ extern "C" int ign_mesh_simplify(ign_mesher* m, const float resolution[3], int r
   if (sl_ctas < 1 || sl_ctas * sl_threads > 1024) sl_ctas = 1024 / sl_threads;
   const size_t sl_static = ((sizeof(SlShared) + 255) / 256) * 256 + 1024;
   const size_t sl_dyn = ((232448 / (size_t)sl_ctas) > sl_static + 16384 ? (232448 / (size_t)sl_ctas) - sl_static : 16384) & ~(size_t)255;
-  S_CUDA(cudaFuncSetAttribute(k_simp_labels, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sl_dyn));
+  IGN_CUDA(cudaFuncSetAttribute(k_simp_labels, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sl_dyn));
   SlArgs A;
   A.pos = s.pos; A.Q = s.Q; A.face = s.face; A.falive = s.falive; A.valive = s.valive; A.vbound = s.vbound;
   A.ecost = ecost; A.key1 = key1; A.fstate = fstate; A.vflag = vflag; A.vlose = vlose;
@@ -1321,11 +1291,11 @@ extern "C" int ign_mesh_simplify(ign_mesher* m, const float resolution[3], int r
   A.trace = nullptr;
   A.lrec = nullptr;
   if (getenv("IGN_SIMP_TRACE") != nullptr) {
-    A.trace = (uint32_t*)scratch_take(ctx, 400 * 16 + 256);
-    A.lrec = (uint32_t*)scratch_take(ctx, (size_t)K * 24 + 64);
+    A.trace = sc.take<uint32_t>(400 * 4 + 64);
+    A.lrec = sc.take<uint32_t>((size_t)K * 6 + 16);
     if (!A.lrec) A.trace = nullptr;
-    if (A.trace) S_CUDA(cudaMemsetAsync(A.trace, 0, 400 * 16 + 256, ctx->stream));
-    if (A.trace) S_CUDA(cudaMemsetAsync(A.lrec, 0, (size_t)K * 24 + 64, ctx->stream));
+    if (A.trace) IGN_CUDA(cudaMemsetAsync(A.trace, 0, 400 * 16 + 256, ctx->stream));
+    if (A.trace) IGN_CUDA(cudaMemsetAsync(A.lrec, 0, (size_t)K * 24 + 64, ctx->stream));
   }
   const char* force_gmem = getenv("IGN_SIMP_GMEM");
   const uint32_t sl_fixed = (uint32_t)((SL_THREADS / 32) * SL_EQ * 4 + SL_WCAP * 2 * S_MAXV * 4);  // queues + ring lists
@@ -1341,35 +1311,35 @@ extern "C" int ign_mesh_simplify(ign_mesher* m, const float resolution[3], int r
     k_simp_labels<<<grid, sl_threads, sl_dyn, ctx->stream>>>(A);
     ctx->launches++;
     prof_end(ctx, slot);
-    S_CUDA(cudaGetLastError());
+    IGN_CUDA(cudaGetLastError());
   }
 
   // ---- compaction
   uint32_t* fscan = node_v;   // 3T u32 >= T
   uint32_t* fflag = node_h;
   size_t tb = tmpb;
-  S_LAUNCH(k_simp_flags_u32, blocks_for(U, 256), 256, s.valive, U, vflag32);
-  S_CUDA(cub::DeviceScan::ExclusiveSum(tmp, tb, vflag32, vscan, (int)U, ctx->stream));
-  S_LAUNCH(k_simp_flags_u32, blocks_for(T, 256), 256, s.falive, T, fflag);
+  IGN_LAUNCH(ctx, k_simp_flags_u32, blocks_for(U, 256), 256, 0, s.valive, U, vflag32);
+  IGN_CUDA(cub::DeviceScan::ExclusiveSum(tmp, tb, vflag32, vscan, (int)U, ctx->stream));
+  IGN_LAUNCH(ctx, k_simp_flags_u32, blocks_for(T, 256), 256, 0, s.falive, T, fflag);
   tb = tmpb;
-  S_CUDA(cub::DeviceScan::ExclusiveSum(tmp, tb, fflag, fscan, (int)T, ctx->stream));
+  IGN_CUDA(cub::DeviceScan::ExclusiveSum(tmp, tb, fflag, fscan, (int)T, ctx->stream));
   ctx->launches += 4;
   uint32_t last[4], hflags[16];
-  S_TRY(small_d2h(ctx, &last[0], vscan + (U - 1), 4));
-  S_TRY(small_d2h(ctx, &last[1], vflag32 + (U - 1), 4));
-  S_TRY(small_d2h(ctx, &last[2], fscan + (T - 1), 4));
-  S_TRY(small_d2h(ctx, &last[3], fflag + (T - 1), 4));
-  S_TRY(small_d2h(ctx, hflags, flags, 64));
-  S_TRY(small_sync(ctx));
+  IGN_TRY(small_d2h(ctx, &last[0], vscan + (U - 1), 4));
+  IGN_TRY(small_d2h(ctx, &last[1], vflag32 + (U - 1), 4));
+  IGN_TRY(small_d2h(ctx, &last[2], fscan + (T - 1), 4));
+  IGN_TRY(small_d2h(ctx, &last[3], fflag + (T - 1), 4));
+  IGN_TRY(small_d2h(ctx, hflags, flags, 64));
+  IGN_TRY(small_sync(ctx));
   if (hflags[12] != 0) {
     set_error("simplify: a vertex has more than %d incident faces", S_VCAP);
-    return done(IGN_ERR_UNSUPPORTED);
+    return IGN_ERR_UNSUPPORTED;
   }
   if (A.trace) {
     std::vector<uint32_t> tr(1600);
-    S_CUDA(cudaMemcpy(tr.data(), A.trace, 1600 * 4, cudaMemcpyDeviceToHost));
+    IGN_CUDA(cudaMemcpy(tr.data(), A.trace, 1600 * 4, cudaMemcpyDeviceToHost));
     unsigned long long phs[10];
-    S_CUDA(cudaMemcpy(phs, A.trace + 1600, 80, cudaMemcpyDeviceToHost));
+    IGN_CUDA(cudaMemcpy(phs, A.trace + 1600, 80, cudaMemcpyDeviceToHost));
     static const char* names[10] = {"P1", "P2 keys", "P3 lose", "P4 select", "setup", "E1 rings", "E2a cost", "E2b flips", "E2c link+collapse", "stop+compact"};
     unsigned long long tot = 0;
     for (int q = 0; q < 10; q++) tot += phs[q];
@@ -1378,7 +1348,7 @@ extern "C" int ign_mesh_simplify(ign_mesher* m, const float resolution[3], int r
     {
       // per-label records: where do the cycles go -- per round (fixed latency) or per face visit?
       std::vector<uint32_t> rec(6 * (size_t)K);
-      S_CUDA(cudaMemcpy(rec.data(), A.lrec, rec.size() * 4, cudaMemcpyDeviceToHost));
+      IGN_CUDA(cudaMemcpy(rec.data(), A.lrec, rec.size() * 4, cudaMemcpyDeviceToHost));
       static const uint32_t edges[] = {0, 500, 1000, 2000, 4000, 8000, 16000, 32000, 64000, 0xFFFFFFFFu};
       fprintf(stderr, "%12s %7s %8s %10s %10s %9s %9s  class(sm/hy/gl)\n", "faces<", "labels", "rounds", "Mcycles", "Mvisits", "kwins", "cyc/round");
       double sr = 0, sv = 0, sc = 0, srr = 0, svv = 0, srv = 0, src = 0, svc = 0;
@@ -1407,17 +1377,17 @@ extern "C" int ign_mesh_simplify(ign_mesher* m, const float resolution[3], int r
   m->simp_labels_smem = hflags[2];
   m->simp_labels_gmem = hflags[3];
   const uint32_t U2 = last[0] + last[1], T2 = last[2] + last[3];
-  S_LAUNCH(k_simp_new_offsets, blocks_for(K + 2, 256), 256, d_vert_off, vscan, (uint32_t)(K + 2), U, U2,
+  IGN_LAUNCH(ctx, k_simp_new_offsets, blocks_for(K + 2, 256), 256, 0, d_vert_off, vscan, (uint32_t)(K + 2), U, U2,
            d_new_vert_off);
-  S_LAUNCH(k_simp_new_offsets, blocks_for(K + 2, 256), 256, d_tri_off, fscan, (uint32_t)(K + 2), T, T2,
+  IGN_LAUNCH(ctx, k_simp_new_offsets, blocks_for(K + 2, 256), 256, 0, d_tri_off, fscan, (uint32_t)(K + 2), T, T2,
            d_new_tri_off);
   // results overwrite the mesher's buffers (inputs were copied into the arena; the vertex buffer holds 12 B / vertex)
   float* pos_f = (float*)m->d_uniq_vkeys;
-  S_LAUNCH(k_simp_compact_verts, blocks_for(U, 256), 256, s, vscan, pos_f);
-  S_LAUNCH(k_simp_compact_faces, blocks_for(T, 256), 256, s, vscan, fscan, d_new_vert_off, m->d_faces);
-  S_TRY(small_d2h(ctx, m->tri_off.data(), d_new_tri_off, (K + 2) * 4));
-  S_TRY(small_d2h(ctx, m->vert_off.data(), d_new_vert_off, (K + 2) * 4));
-  S_TRY(small_sync(ctx));
+  IGN_LAUNCH(ctx, k_simp_compact_verts, blocks_for(U, 256), 256, 0, s, vscan, pos_f);
+  IGN_LAUNCH(ctx, k_simp_compact_faces, blocks_for(T, 256), 256, 0, s, vscan, fscan, d_new_vert_off, m->d_faces);
+  IGN_TRY(small_d2h(ctx, m->tri_off.data(), d_new_tri_off, (K + 2) * 4));
+  IGN_TRY(small_d2h(ctx, m->vert_off.data(), d_new_vert_off, (K + 2) * 4));
+  IGN_TRY(small_sync(ctx));
   m->U = U2;
   m->T = T2;
   m->d_pos_f = pos_f;
@@ -1425,5 +1395,5 @@ extern "C" int ign_mesh_simplify(ign_mesher* m, const float resolution[3], int r
   m->present.clear();
   for (uint64_t l = 1; l <= K; l++)
     if (m->tri_off[l + 1] > m->tri_off[l]) m->present.push_back(m->ids[l - 1]);
-  return done(IGN_OK);
+  return IGN_OK;
 }
